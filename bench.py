@@ -2,6 +2,7 @@
 """bench.py -- guided scenarios/s of the CLD sampling hot path on B200 (contract in the task brief).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config cfg1|cfg2|cfg3|cfg4] [--precision bf16|fp32]
+                  [--dump-outputs DIR]
 
 A "step" = ONE pass of the hot path over one batch of synthetic nuScenes-shaped scenes:
     S scenes x A agents x N samples  ->  K_d denoising steps (denoiser + posterior update [+ guidance])
@@ -69,7 +70,13 @@ def parse():
     ap.add_argument("--skip-lanes", action="store_true", help="same as --lanes 1 (one engine / stream; the kernel brackets then come from the timed region)")
     ap.add_argument("--skip-context", action="store_true", help="do not time the context encoder (row a14) after the headline")
     ap.add_argument("--skip-hbm", action="store_true", help="do not time the HBM-bound kernels (K3, K6) alone")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (see dump_outputs)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.warmup < 0:
+        ap.error("--warmup must not be negative")
     a.w = dict(WORKLOADS[a.config])
     if a.sampler:
         a.w["sampler"] = a.sampler
@@ -217,12 +224,41 @@ def cpu_oracle_rate(a, n_scenes, steps, warmup):
     return n_scenes / dt, dt, cores, c, res, den_rows_s
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(d, arrays):
+    """Writes the tensors of `arrays` (name -> tensor; nested dicts as "<outer>.<inner>") to d/<name>.npy, float64 and 32/64-bit
+    integer tensors as float64 (float32 cannot hold all their values), everything else as float32, so that the results of two builds
+    can be compared output for output.  Above DUMP_BYTES in all, every array keeps the same fraction of its rows (leading dimension),
+    chosen by a fixed seed: two runs with the same arguments write the same rows."""
+    import numpy as np
+    import torch
+    flat = {}
+    for k, v in arrays.items():
+        for k2, v2 in (v.items() if isinstance(v, dict) else [(None, v)]):
+            if torch.is_tensor(v2):
+                flat[k if k2 is None else "%s.%s" % (k, k2)] = v2
+    wide = lambda v: v.dtype in (torch.float64, torch.int32, torch.int64)   # noqa: E731
+    total = sum(v.numel() * (8 if wide(v) else 4) for v in flat.values())
+    frac = min(1.0, DUMP_BYTES / max(total, 1))
+    os.makedirs(d, exist_ok=True)
+    for k, v in sorted(flat.items()):
+        if frac < 1.0 and v.dim() > 0:
+            keep = torch.randperm(v.shape[0], generator=torch.Generator().manual_seed(0))[:max(1, int(v.shape[0] * frac))]
+            v = v.index_select(0, keep.sort().values.to(v.device))
+        v = v.detach().to("cpu", torch.float64 if wide(v) else torch.float32)
+        np.save(os.path.join(d, k + ".npy"), v.numpy())
+
+
 def run_reference(a):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warm = max(1, min(a.steps, 3)), min(max(a.warmup, 0), 1)
-    rate, dt, cores, _, _, den = cpu_oracle_rate(a, a.cpu_scenes, steps, warm)
+    steps, warm = a.steps, a.warmup
+    rate, dt, cores, _, res, den = cpu_oracle_rate(a, a.cpu_scenes, steps, warm)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, dict(zip(("pred_traj", "traj", "offroad", "coll"), res)))
     sample = "%d of %d scenes of %s, oracle port of the reference's PyTorch sampler (guidance through autograd as in the reference), %d host threads" % (
         a.cpu_scenes, a.w["scenes"], workload_text(a), cores)
     print(json.dumps({
@@ -504,6 +540,8 @@ def main():
     launches = count_launches() - l0
     clocks = sampler_thread.stop() if sampler_thread else None
     ms = e0.elapsed_time(e1) / a.steps
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, out)
     single = None
     if n_lanes > 1:
         # the same workload on ONE engine / stream, per-kind CUDA-event brackets around every kernel group: each kernel is timed alone
