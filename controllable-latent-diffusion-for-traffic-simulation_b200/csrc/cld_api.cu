@@ -44,7 +44,7 @@ int prof_end(CldHandle* h, cudaStream_t s) {
 
 template <typename T>
 static int dev_alloc(CldHandle* h, T** p, size_t n) {
-  if (*p) return 0;      // re-load of the weights (every optimizer step of the PPO update): sizes are fixed by the config, reuse
+  if (*p) return 0;      // re-load of the decoder weights: sizes are fixed by the config, reuse
   void* q = nullptr;
   CLD_CUDA_OK(h, cudaMalloc(&q, (n ? n : 1) * sizeof(T)));
   h->allocs.push_back(q);
@@ -52,33 +52,9 @@ static int dev_alloc(CldHandle* h, T** p, size_t n) {
   return 0;
 }
 
-// dst[(tap*cin + ci)*ld + off + co] = src[co, ci, k(tap)]  (Conv1d / Linear weights, [cout][cin][K])
-// transposed=1: src is ConvTranspose1d weight [cin][cout][K]
-__global__ void pack_conv_kernel(const float* __restrict__ src, float* __restrict__ dst, int cout, int cin, int K,
-                                 int ntaps, int k0, int k1, int k2, int k3, int k4, int ld, int off, int transposed) {
-  int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  int total = ntaps * cin * cout;
-  if (idx >= total) return;
-  int co = idx % cout, ci = (idx / cout) % cin, tap = idx / (cout * cin);
-  int ks[5] = {k0, k1, k2, k3, k4};
-  int k = ks[tap];
-  float v = transposed ? src[((size_t)ci * cout + co) * K + k] : src[((size_t)co * cin + ci) * K + k];
-  dst[((size_t)tap * cin + ci) * ld + off + co] = v;
-}
-
-// dst[(tap*cout + co)*cin + ci] = src[co, ci, k(tap)]: the [N][K] (K contiguous) weight planes of the tensor-core training forward
-__global__ void pack_conv_t_kernel(const float* __restrict__ src, float* __restrict__ dst, int cout, int cin, int K, int ntaps,
-                                   int k0, int k1, int k2, int k3, int k4, int transposed) {
-  int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  int total = ntaps * cin * cout;
-  if (idx >= total) return;
-  int ci = idx % cin, co = (idx / cin) % cout, tap = idx / (cout * cin);
-  int ks[5] = {k0, k1, k2, k3, k4};
-  dst[idx] = transposed ? src[((size_t)ci * cout + co) * K + ks[tap]] : src[((size_t)co * cin + ci) * K + ks[tap]];
-}
-
-// ---- fused re-pack: all pack / copy jobs of cld_load_unet in ONE launch (the weights change after every optimizer step)
-struct PackSrc { const float* p[160]; };
+// ---- weight pack: every pack / copy job of cld_load_unet in ONE launch (the weights change after every optimizer step)
+constexpr int PACK_MAX_SRC = 160;
+struct PackSrc { const float* p[PACK_MAX_SRC]; };
 constexpr int PACK_BLOCK_ELEMS = 2048;
 __global__ void __launch_bounds__(256) repack_all_kernel(const PackJob* __restrict__ jobs, int njobs, PackSrc src) {
   int lo = 0, hi = njobs - 1;                       // last job whose first block is <= blockIdx.x
@@ -103,20 +79,6 @@ __global__ void __launch_bounds__(256) repack_all_kernel(const PackJob* __restri
   }
 }
 
-static void record_job(CldHandle* h, int kind, const float* src, float* dst, int cout, int cin, int K, int ntaps, const int* ks, int ld,
-                       int off, int transposed, int total) {
-  if (!h->pack_recording) return;
-  int si = -1;
-  for (int i = 0; i < h->pack_nsrc; ++i)
-    if (h->pack_src[i] == src) { si = i; break; }
-  if (si < 0) { h->pack_recording = false; h->pack_jobs.clear(); return; }      // a source outside the list: no fast path
-  PackJob j;
-  j.kind = kind; j.src = si; j.dst = dst; j.cout = cout; j.cin = cin; j.K = K; j.ntaps = ntaps;
-  for (int i = 0; i < 5; ++i) j.ks[i] = (ks && i < ntaps) ? ks[i] : 0;
-  j.ld = ld; j.off = off; j.transposed = transposed; j.total = total; j.blk0 = 0;
-  h->pack_jobs.push_back(j);
-}
-
 __global__ void transpose_kernel(const float* __restrict__ src, float* __restrict__ dst, int rows, int cols) {
   int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= rows * cols) return;
@@ -133,25 +95,122 @@ static int copy_vec(CldHandle* h, float** dst, const float* src, size_t n, cudaS
   int rc = dev_alloc(h, dst, n);
   if (rc) return rc;
   CLD_CUDA_OK(h, cudaMemcpyAsync(*dst, src, n * sizeof(float), cudaMemcpyDeviceToDevice, s));
-  record_job(h, 2, src, *dst, 0, 0, 0, 0, nullptr, 0, 0, 0, (int)n);
   return 0;
 }
 
-static int pack_conv(CldHandle* h, ConvW* w, const float* src, const float* bias, int cout, int cin, int K,
-                     int ntaps, const int* ks, int transposed, cudaStream_t s) {
-  int rc;
-  w->cin = cin; w->cout = cout; w->ntaps = ntaps;
-  if ((rc = dev_alloc(h, &w->w, (size_t)ntaps * cin * cout))) return rc;
-  int total = ntaps * cin * cout;
-  pack_conv_kernel<<<(total + 255) / 256, 256, 0, s>>>(src, w->w, cout, cin, K, ntaps, ks[0], ks[1], ks[2], ks[3], ks[4],
-                                                       cout, 0, transposed);
-  CLD_LAUNCH_OK(h, "pack_conv_kernel");
-  record_job(h, 0, src, w->w, cout, cin, K, ntaps, ks, cout, 0, transposed, total);
-  if ((rc = dev_alloc(h, &w->wt, (size_t)ntaps * cin * cout))) return rc;
-  pack_conv_t_kernel<<<(total + 255) / 256, 256, 0, s>>>(src, w->wt, cout, cin, K, ntaps, ks[0], ks[1], ks[2], ks[3], ks[4], transposed);
-  CLD_LAUNCH_OK(h, "pack_conv_t_kernel");
-  record_job(h, 1, src, w->wt, cout, cin, K, ntaps, ks, 0, 0, transposed, total);
-  if (bias) return copy_vec(h, &w->b, bias, cout, s);
+// Channels of the residual blocks in execution order (downs.{0,1,2}.{0,1}, mid_block1, mid_block2, ups.{0,1}.{0,1}) and their slices of
+// the concatenated time-bias, in the same order.
+static void unet_blocks(UnetW& u, const CldConfig& c) {
+  const int D = c.latent_dim, d0 = c.dims[0], d1 = c.dims[1], d2 = c.dims[2];
+  const int in_ch[12] = {D, d0, d0, d1, d1, d2, d2, d2, 2 * d2, d1, 2 * d1, d0};
+  const int out_ch[12] = {d0, d0, d1, d1, d2, d2, d2, d2, d1, d1, d0, d0};
+  for (int e = 0; e < 12; ++e) {
+    u.rb[e].cin = in_ch[e]; u.rb[e].cout = out_ch[e]; u.rb[e].tb_off = u.tb_total;
+    u.tb_total += out_ch[e];
+  }
+}
+
+// The denoiser's state-dict layout (DmModel.model.state_dict(), temporal.py:49-120), its packed fp32 buffers and the pack table that
+// fills them from the state-dict tensors: one walk over the module tree in state-dict order (after unet_blocks).  Depends on the
+// config only.
+static int unet_setup(CldHandle* h) {
+  const CldConfig& c = h->cfg;
+  const int d = c.base_dim, D = c.latent_dim, tdim = c.base_dim + c.cond_dim;
+  const int d0 = c.dims[0], d1 = c.dims[1];
+  UnetW& u = h->unet;
+  UnetLayout& L = h->unet_layout;
+  const int k5[5] = {0, 1, 2, 3, 4}, k3[5] = {0, 1, 2, 0, 0}, k1[5] = {0, 0, 0, 0, 0};
+  const int kte[5] = {1, 3, 0, 0, 0}, kto[5] = {0, 2, 0, 0, 0};   // transposed conv: taps of the even / odd output phase
+  std::vector<PackJob> jobs;
+  int rc = 0;
+  auto buf = [&](float** p, size_t n) { if (!rc) rc = dev_alloc(h, p, n); return *p; };
+  auto take = [&](int64_t numel) { L.numel.push_back(numel); return (int)L.numel.size() - 1; };
+  auto job = [&](int kind, int src, float* dst, int total) -> PackJob& {
+    PackJob j = {};
+    j.kind = kind; j.src = src; j.dst = dst; j.total = total;
+    jobs.push_back(j);
+    return jobs.back();
+  };
+  auto vec = [&](float** dst, int n) { const int i = take(n); job(2, i, buf(dst, n), n); return i; };
+  // weight `src` [cout][cin][K] (transposed: [cin][cout][K]), taps ks: -> w [tap][cin][cout] and wt [tap][cout][cin]
+  auto pack = [&](ConvW& w, int src, int cout, int cin, int K, int ntaps, const int* ks, int transposed) {
+    w.cin = cin; w.cout = cout; w.ntaps = ntaps;
+    for (int kind = 0; kind < 2; ++kind) {
+      PackJob& j = job(kind, src, buf(kind ? &w.wt : &w.w, (size_t)ntaps * cin * cout), ntaps * cin * cout);
+      j.cout = cout; j.cin = cin; j.K = K; j.ntaps = ntaps; j.ld = kind ? 0 : cout; j.transposed = transposed;
+      for (int t = 0; t < ntaps; ++t) j.ks[t] = ks[t];
+    }
+  };
+  auto conv = [&](ConvW& w, int cout, int cin, int K, const int* ks, int& iw, int& ib) {
+    iw = take((int64_t)cout * cin * K);
+    ib = take(cout);
+    pack(w, iw, cout, cin, K, K, ks, 0);
+    job(2, ib, buf(&w.b, cout), cout);
+  };
+  auto block = [&](int e) {
+    ResBlockW& rb = u.rb[e];
+    BlkIdx& b = L.blk[e];
+    b.tw = take((int64_t)rb.cout * tdim);
+    b.tb = take(rb.cout);
+    PackJob& j = job(0, b.tw, u.tb_w, rb.cout * tdim);    // time / cond projection: columns tb_off .. tb_off + cout of [tdim][tb_total]
+    j.cout = rb.cout; j.cin = tdim; j.K = 1; j.ntaps = 1; j.ld = u.tb_total; j.off = rb.tb_off;
+    job(2, b.tb, u.tb_b + rb.tb_off, rb.cout);
+    // torch's Linear weight [cout][tdim] IS the [N][K] plane the tensor-core training forward reads: rows tb_off .. tb_off + cout
+    job(2, b.tw, u.tb_wt + (size_t)rb.tb_off * tdim, rb.cout * tdim);
+    conv(rb.c0, rb.cout, rb.cin, 5, k5, b.c0w, b.c0b);
+    b.g0 = vec(&rb.n0.g, rb.cout);
+    b.b0 = vec(&rb.n0.b, rb.cout);
+    conv(rb.c1, rb.cout, rb.cout, 5, k5, b.c1w, b.c1b);
+    b.g1 = vec(&rb.n1.g, rb.cout);
+    b.b1 = vec(&rb.n1.b, rb.cout);
+    b.rw = b.rb = -1;
+    if (rb.cin != rb.cout) conv(rb.res, rb.cout, rb.cin, 1, k1, b.rw, b.rb);
+  };
+  L.tmlp[0] = vec(&u.t1_w, 4 * d * d);
+  L.tmlp[1] = vec(&u.t1_b, 4 * d);
+  L.tmlp[2] = vec(&u.t2_w, 4 * d * d);
+  L.tmlp[3] = vec(&u.t2_b, d);
+  {
+    // SinusoidalPosEmb frequencies, same fp32 op order as the reference (diffuser_helpers.py:27-29)
+    std::vector<float> f(d / 2);
+    double emb = log(10000.0) / (double)(d / 2 - 1);
+    for (int i = 0; i < d / 2; ++i) f[i] = expf((float)i * (float)(-emb));
+    if (buf(&u.freqs, d / 2)) CLD_CUDA_OK(h, cudaMemcpy(u.freqs, f.data(), f.size() * sizeof(float), cudaMemcpyHostToDevice));
+  }
+  buf(&u.tb_w, (size_t)tdim * u.tb_total);
+  buf(&u.tb_b, u.tb_total);
+  buf(&u.tb_wt, (size_t)tdim * u.tb_total);
+  for (int lvl = 0; lvl < 3; ++lvl) {             // downs.lvl: two blocks, then Downsample1d (not on the last level)
+    block(2 * lvl);
+    block(2 * lvl + 1);
+    if (lvl < 2) conv(u.down[lvl], c.dims[lvl], c.dims[lvl], 3, k3, L.down[lvl][0], L.down[lvl][1]);
+  }
+  for (int lvl = 0; lvl < 2; ++lvl) {             // ups.lvl: two blocks, then Upsample1d (ConvTranspose1d k4 s2 p1)
+    block(8 + 2 * lvl);
+    block(9 + 2 * lvl);
+    const int ch = lvl == 0 ? d1 : d0;
+    const int iw = L.up[lvl][0] = take((int64_t)ch * ch * 4), ib = L.up[lvl][1] = take(ch);
+    pack(u.up[lvl][0], iw, ch, ch, 4, 2, kte, 1);
+    pack(u.up[lvl][1], iw, ch, ch, 4, 2, kto, 1);
+    job(2, ib, buf(&u.up_b[lvl], ch), ch);
+  }
+  block(6);                                       // mid_block1, mid_block2
+  block(7);
+  conv(u.fin0, d0, d0, 5, k5, L.fin[0], L.fin[1]);   // final_conv: Conv1dBlock(d0, d0, 5), Conv1d(d0, D, 1)
+  L.fin[2] = vec(&u.fin0n.g, d0);
+  L.fin[3] = vec(&u.fin0n.b, d0);
+  conv(u.fin1, D, d0, 1, k1, L.fin[4], L.fin[5]);
+  if (rc) return rc;
+  if (L.numel.size() > (size_t)PACK_MAX_SRC)
+    return fail(h, CLD_ERR_UNSUPPORTED, "the denoiser has %zu tensors, the weight pack takes at most %d", L.numel.size(), PACK_MAX_SRC);
+  for (PackJob& j : jobs) {
+    j.blk0 = h->pack_blocks;
+    h->pack_blocks += (j.total + PACK_BLOCK_ELEMS - 1) / PACK_BLOCK_ELEMS;
+  }
+  h->pack_njobs = (int)jobs.size();
+  if ((rc = dev_alloc(h, &h->pack_jobs, jobs.size()))) return rc;
+  CLD_CUDA_OK(h, cudaMemcpy(h->pack_jobs, jobs.data(), jobs.size() * sizeof(PackJob), cudaMemcpyHostToDevice));
+  CLD_CUDA_OK(h, cudaStreamSynchronize(cudaStreamLegacy));   // pageable uploads: complete before any stream of the caller reads them
   return 0;
 }
 
@@ -213,8 +272,8 @@ int cld_create(const CldConfig* cfg, CldHandle** out) {
   if ((size_t)(T / 2) * cfg->dims[1] > ae) ae = (size_t)(T / 2) * cfg->dims[1];
   if ((size_t)(T / 4) * cfg->dims[2] > ae) ae = (size_t)(T / 4) * cfg->dims[2];
   h->act_elems = ae;
-  int tb_total = 2 * (cfg->dims[0] + cfg->dims[1] + cfg->dims[2]) + 2 * cfg->dims[2] + 2 * cfg->dims[1] + 2 * cfg->dims[0];
-  h->unet.tb_total = tb_total;
+  unet_blocks(h->unet, *cfg);
+  const int tb_total = h->unet.tb_total;
   int rc = 0;
   for (int i = 0; i < 7 && !rc; ++i) rc = dev_alloc(h, &h->act[i], MR * ae);
   if (!rc) rc = dev_alloc(h, &h->tcm, MR * (cfg->base_dim + cfg->cond_dim));
@@ -236,6 +295,7 @@ int cld_create(const CldConfig* cfg, CldHandle** out) {
   if (!rc) rc = dev_alloc(h, &h->ws_mean, MR * T * cfg->latent_dim);
   if (!rc) rc = dev_alloc(h, &h->ws_x, MR * T * cfg->latent_dim);
   if (!rc) rc = dev_alloc(h, &h->ws_t, MR);
+  if (!rc) rc = unet_setup(h);
   if (rc) {
     g_create_err = h->err;
     cld_destroy(h);
@@ -262,152 +322,23 @@ void cld_destroy(CldHandle* h) {
 
 int cld_load_unet(CldHandle* h, const float* const* p, const int64_t* numels, int n, void* stream) {
   if (!h || !p) return fail(h, CLD_ERR_ARG, "null argument");
+  const UnetLayout& L = h->unet_layout;
+  if (n != (int)L.numel.size()) return fail(h, CLD_ERR_ARG, "cld_load_unet: expected %zu tensors, got %d", L.numel.size(), n);
+  PackSrc src;
+  for (int i = 0; i < n; ++i) {
+    if (!p[i]) return fail(h, CLD_ERR_ARG, "cld_load_unet: tensor %d is null", i);
+    if (numels && numels[i] != L.numel[i])
+      return fail(h, CLD_ERR_ARG, "cld_load_unet: tensor %d has %lld elements, expected %lld", i, (long long)numels[i], (long long)L.numel[i]);
+    src.p[i] = p[i];
+  }
   cudaStream_t s = (cudaStream_t)stream;
-  const CldConfig& c = h->cfg;
-  const int d = c.base_dim, D = c.latent_dim, tdim = c.base_dim + c.cond_dim;
-  const int d0 = c.dims[0], d1 = c.dims[1], d2 = c.dims[2];
-  // residual blocks in STATE-DICT order: downs.{0,1,2}.{0,1}, ups.{0,1}.{0,1}, mid_block1, mid_block2
-  struct BlkDef { int cin, cout, exec; };
-  const BlkDef defs[12] = {{D, d0, 0}, {d0, d0, 1}, {d0, d1, 2}, {d1, d1, 3}, {d1, d2, 4}, {d2, d2, 5},
-                           {2 * d2, d1, 8}, {d1, d1, 9}, {2 * d1, d0, 10}, {d0, d0, 11}, {d2, d2, 6}, {d2, d2, 7}};
-  // expected tensor count
-  int expect = 4;
-  for (int b = 0; b < 12; ++b) expect += 10 + (defs[b].cin != defs[b].cout ? 2 : 0);
-  expect += 2 * 2 + 2 * 2 + 4 + 2;
-  if (n != expect) return fail(h, CLD_ERR_ARG, "cld_load_unet: expected %d tensors, got %d", expect, n);
-  int idx = 0, rc;
-  UnetW& u = h->unet;
-  // ---- re-load of a loaded fp32 handle (every optimizer step of the PPO update): ONE launch instead of ~80 pack kernels + ~100 copies
-  if (u.loaded && !tc_enabled(h) && h->pack_jobs_dev && n <= 160) {
-    PackSrc src;
-    for (int i = 0; i < n; ++i) {
-      if (!p[i]) return fail(h, CLD_ERR_ARG, "cld_load_unet: tensor %d is null", i);
-      src.p[i] = p[i];
-    }
-    repack_all_kernel<<<h->pack_blocks, 256, 0, s>>>(h->pack_jobs_dev, (int)h->pack_jobs.size(), src);
-    CLD_LAUNCH_OK(h, "repack_all_kernel");
-    h->tvec_all_valid = false;
-    train_invalidate(h);
-    return CLD_OK;
-  }
-  h->pack_jobs.clear();
-  h->pack_recording = !tc_enabled(h) && n <= 160;
-  h->pack_src = p; h->pack_nsrc = n;
-  auto chk = [&](int i, int64_t want) -> bool { return !numels || numels[i] == want; };
-#define NEXT(want)                                                                                        \
-  (chk(idx, (int64_t)(want)) ? p[idx++]                                                                   \
-                             : (fail(h, CLD_ERR_ARG, "cld_load_unet: tensor %d has %lld elements, expected %lld", idx, \
-                                     (long long)numels[idx], (long long)(want)),                          \
-                                (const float*)nullptr))
-#define TAKE(var, want)            \
-  const float* var = NEXT(want);   \
-  if (!var) return CLD_ERR_ARG;
-  TAKE(t1w, 4 * d * d) TAKE(t1b, 4 * d) TAKE(t2w, d * 4 * d) TAKE(t2b, d)
-  if ((rc = copy_vec(h, &u.t1_w, t1w, 4 * d * d, s))) return rc;
-  if ((rc = copy_vec(h, &u.t1_b, t1b, 4 * d, s))) return rc;
-  if ((rc = copy_vec(h, &u.t2_w, t2w, 4 * d * d, s))) return rc;
-  if ((rc = copy_vec(h, &u.t2_b, t2b, d, s))) return rc;
-  {
-    // SinusoidalPosEmb frequencies, same fp32 op order as the reference (diffuser_helpers.py:27-29)
-    std::vector<float> f(d / 2);
-    double emb = log(10000.0) / (double)(d / 2 - 1);
-    for (int i = 0; i < d / 2; ++i) f[i] = expf((float)i * (float)(-emb));
-    if ((rc = dev_alloc(h, &u.freqs, d / 2))) return rc;
-    CLD_CUDA_OK(h, cudaMemcpyAsync(u.freqs, f.data(), f.size() * sizeof(float), cudaMemcpyHostToDevice, s));
-    CLD_CUDA_OK(h, cudaStreamSynchronize(s));
-  }
-  if ((rc = dev_alloc(h, &u.tb_w, (size_t)tdim * u.tb_total))) return rc;
-  if ((rc = dev_alloc(h, &u.tb_b, u.tb_total))) return rc;
-  if ((rc = dev_alloc(h, &u.tb_wt, (size_t)tdim * u.tb_total))) return rc;
-  // time-bias offsets follow EXECUTION order
-  int exec_cout[12];
-  for (int b = 0; b < 12; ++b) exec_cout[defs[b].exec] = defs[b].cout;
-  int exec_off[12], acc = 0;
-  for (int e = 0; e < 12; ++e) { exec_off[e] = acc; acc += exec_cout[e]; }
-  const int k5[5] = {0, 1, 2, 3, 4}, k1[5] = {0, 0, 0, 0, 0}, k3[5] = {0, 1, 2, 0, 0};
-  const int kte[5] = {1, 3, 0, 0, 0}, kto[5] = {0, 2, 0, 0, 0};
-  auto load_block = [&](const BlkDef& bd) -> int {
-    ResBlockW& rb = u.rb[bd.exec];
-    rb.cin = bd.cin; rb.cout = bd.cout; rb.tb_off = exec_off[bd.exec];
-    TAKE(tw, bd.cout * tdim) TAKE(tbv, bd.cout)
-    {
-      int total = tdim * bd.cout;
-      pack_conv_kernel<<<(total + 255) / 256, 256, 0, s>>>(tw, u.tb_w, bd.cout, tdim, 1, 1, 0, 0, 0, 0, 0, u.tb_total,
-                                                           rb.tb_off, 0);
-      CLD_LAUNCH_OK(h, "pack_conv_kernel");
-      CLD_CUDA_OK(h, cudaMemcpyAsync(u.tb_b + rb.tb_off, tbv, bd.cout * sizeof(float), cudaMemcpyDeviceToDevice, s));
-      const int k1x[5] = {0, 0, 0, 0, 0};
-      record_job(h, 0, tw, u.tb_w, bd.cout, tdim, 1, 1, k1x, u.tb_total, rb.tb_off, 0, total);
-      record_job(h, 2, tbv, u.tb_b + rb.tb_off, 0, 0, 0, 0, nullptr, 0, 0, 0, bd.cout);
-      // torch's Linear weight [cout][tdim] IS the [N][K] plane the tensor-core training forward reads: rows tb_off .. tb_off + cout
-      CLD_CUDA_OK(h, cudaMemcpyAsync(u.tb_wt + (size_t)rb.tb_off * tdim, tw, (size_t)bd.cout * tdim * sizeof(float), cudaMemcpyDeviceToDevice, s));
-      record_job(h, 2, tw, u.tb_wt + (size_t)rb.tb_off * tdim, 0, 0, 0, 0, nullptr, 0, 0, 0, bd.cout * tdim);
-    }
-    TAKE(c0w, bd.cout * bd.cin * 5) TAKE(c0b, bd.cout) TAKE(g0, bd.cout) TAKE(b0, bd.cout)
-    TAKE(c1w, bd.cout * bd.cout * 5) TAKE(c1b, bd.cout) TAKE(g1, bd.cout) TAKE(b1, bd.cout)
-    int r;
-    if ((r = pack_conv(h, &rb.c0, c0w, c0b, bd.cout, bd.cin, 5, 5, k5, 0, s))) return r;
-    if ((r = copy_vec(h, &rb.n0.g, g0, bd.cout, s))) return r;
-    if ((r = copy_vec(h, &rb.n0.b, b0, bd.cout, s))) return r;
-    if ((r = pack_conv(h, &rb.c1, c1w, c1b, bd.cout, bd.cout, 5, 5, k5, 0, s))) return r;
-    if ((r = copy_vec(h, &rb.n1.g, g1, bd.cout, s))) return r;
-    if ((r = copy_vec(h, &rb.n1.b, b1, bd.cout, s))) return r;
-    if (bd.cin != bd.cout) {
-      TAKE(rw, bd.cout * bd.cin) TAKE(rbv, bd.cout)
-      if ((r = pack_conv(h, &rb.res, rw, rbv, bd.cout, bd.cin, 1, 1, k1, 0, s))) return r;
-    }
-    if (tc_enabled(h) && (r = tc_pack_block(h, bd.exec, bd.cin, bd.cout, c0w, c0b, g0, b0, c1w, c1b, g1, b1,
-                                            bd.cin != bd.cout ? p[idx - 2] : nullptr,
-                                            bd.cin != bd.cout ? p[idx - 1] : nullptr, s)))
-      return r;
-    return 0;
-  };
-  // downs
-  for (int lvl = 0; lvl < 3; ++lvl) {
-    if ((rc = load_block(defs[lvl * 2]))) return rc;
-    if ((rc = load_block(defs[lvl * 2 + 1]))) return rc;
-    if (lvl < 2) {
-      int ch = c.dims[lvl];
-      TAKE(dw, ch * ch * 3) TAKE(db, ch)
-      if ((rc = pack_conv(h, &u.down[lvl], dw, db, ch, ch, 3, 3, k3, 0, s))) return rc;
-      if (tc_enabled(h) && (rc = tc_pack_down(h, lvl, ch, dw, db, s))) return rc;
-    }
-  }
-  // ups
-  for (int lvl = 0; lvl < 2; ++lvl) {
-    if ((rc = load_block(defs[6 + lvl * 2]))) return rc;
-    if ((rc = load_block(defs[6 + lvl * 2 + 1]))) return rc;
-    int ch = lvl == 0 ? d1 : d0;
-    TAKE(uw, ch * ch * 4) TAKE(ub, ch)
-    if ((rc = pack_conv(h, &u.up[lvl][0], uw, nullptr, ch, ch, 4, 2, kte, 1, s))) return rc;
-    if ((rc = pack_conv(h, &u.up[lvl][1], uw, nullptr, ch, ch, 4, 2, kto, 1, s))) return rc;
-    if ((rc = copy_vec(h, &u.up_b[lvl], ub, ch, s))) return rc;
-    if (tc_enabled(h) && (rc = tc_pack_up(h, lvl, ch, uw, ub, s))) return rc;
-  }
-  if ((rc = load_block(defs[10]))) return rc;
-  if ((rc = load_block(defs[11]))) return rc;
-  {
-    TAKE(fw, d0 * d0 * 5) TAKE(fb, d0) TAKE(fg, d0) TAKE(fbt, d0) TAKE(f1w, D * d0) TAKE(f1b, D)
-    if ((rc = pack_conv(h, &u.fin0, fw, fb, d0, d0, 5, 5, k5, 0, s))) return rc;
-    if ((rc = copy_vec(h, &u.fin0n.g, fg, d0, s))) return rc;
-    if ((rc = copy_vec(h, &u.fin0n.b, fbt, d0, s))) return rc;
-    if ((rc = pack_conv(h, &u.fin1, f1w, f1b, D, d0, 1, 1, k1, 0, s))) return rc;
-    if (tc_enabled(h) && (rc = tc_pack_final(h, fw, fb, fg, fbt, f1w, f1b, s))) return rc;
-  }
-#undef TAKE
-#undef NEXT
-  if (tc_enabled(h) && (rc = tc_finalize(h, s))) return rc;
-  if (h->pack_recording && !h->pack_jobs.empty()) {
-    int blk = 0;
-    for (PackJob& j : h->pack_jobs) { j.blk0 = blk; blk += (j.total + PACK_BLOCK_ELEMS - 1) / PACK_BLOCK_ELEMS; }
-    h->pack_blocks = blk;
-    if ((rc = dev_alloc(h, &h->pack_jobs_dev, h->pack_jobs.size()))) return rc;
-    CLD_CUDA_OK(h, cudaMemcpyAsync(h->pack_jobs_dev, h->pack_jobs.data(), h->pack_jobs.size() * sizeof(PackJob), cudaMemcpyHostToDevice, s));
-  }
-  h->pack_recording = false; h->pack_src = nullptr;
-  CLD_CUDA_OK(h, cudaStreamSynchronize(s));
-  u.loaded = true;
+  repack_all_kernel<<<h->pack_blocks, 256, 0, s>>>(h->pack_jobs, h->pack_njobs, src);
+  CLD_LAUNCH_OK(h, "repack_all_kernel");
   h->tvec_all_valid = false;
+  train_invalidate(h);
+  int rc;
+  if (h->cfg.precision == CLD_PREC_BF16 && (rc = tc_finalize(h, p, s))) return rc;
+  h->unet.loaded = true;
   return CLD_OK;
 }
 

@@ -75,7 +75,18 @@ struct Schedule {
 }  // namespace cld
 
 namespace cld {
-// one entry of the fused weight re-pack (cld_load_unet on a handle that is already loaded: every optimizer step of the PPO update)
+// State-dict layout of the denoiser: the tensors of DmModel.model.state_dict() that cld_load_unet takes and cld_unet_backward writes,
+// by index.  Depends on the config only (built at cld_create).
+struct BlkIdx { int tw, tb, c0w, c0b, g0, b0, c1w, c1b, g1, b1, rw, rb; };   // rw = rb = -1: identity residual
+struct UnetLayout {
+  std::vector<int64_t> numel;   // element count of every state-dict tensor
+  int tmlp[4];                  // time_mlp: Linear(d, 4d) weight, bias; Linear(4d, d) weight, bias
+  BlkIdx blk[12];               // residual blocks in execution order (UnetW::rb)
+  int down[2][2], up[2][2];     // {weight, bias} of the down / up convolutions
+  int fin[6];                   // final_conv: conv weight, bias, GroupNorm weight, bias; 1x1 conv weight, bias
+};
+
+// one entry of the weight pack table: cld_load_unet packs all of them in one launch
 struct PackJob {
   int kind;            // 0: conv [cout][cin][K] -> [tap][cin][ld] (+off); 1: -> [tap][cout][cin]; 2: flat copy
   int src;             // index into the state-dict pointer list
@@ -90,6 +101,7 @@ struct CldHandle {
   int num_sms = 0;
   std::string err;
   cld::UnetW unet;
+  cld::UnetLayout unet_layout;
   cld::DecoderW dec;
   cld::Schedule sched;
   std::vector<void*> allocs;       // everything cudaMalloc'ed by the handle
@@ -145,13 +157,9 @@ struct CldHandle {
   // denoiser training state (opaque, owned by kernels_unet_train.cu): activation stash + gradient scratch, allocated on first use
   void* train = nullptr;
   unsigned long long sched_version = 0;   // bumped by cld_set_schedule
-  // fused re-pack: the jobs recorded during the first cld_load_unet, and their device copy
-  std::vector<cld::PackJob> pack_jobs;
-  cld::PackJob* pack_jobs_dev = nullptr;
-  int pack_blocks = 0;
-  bool pack_recording = false;
-  const float* const* pack_src = nullptr;
-  int pack_nsrc = 0;
+  // the pack table cld_load_unet launches (device copy, built at cld_create), and the grid it needs
+  cld::PackJob* pack_jobs = nullptr;
+  int pack_njobs = 0, pack_blocks = 0;
   void* train_tc = nullptr;        // tensor-map cache of the tf32 tensor-core convolutions (train_tc.cu)
   bool train_tf32 = false;         // cld_train_set_precision: stride-1 convolutions of the training step on the tensor pipe
   // debug switches, read from the environment ONCE at cld_create (never inside the step path)

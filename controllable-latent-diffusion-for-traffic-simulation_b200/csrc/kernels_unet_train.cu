@@ -614,7 +614,6 @@ __global__ void adam_tick_kernel(long long* __restrict__ step, const double* __r
 // host side
 // ------------------------------------------------------------------------------------------------
 struct BlkStash { const float* in0; int c0; const float* in1; int c1; int T; float *A0, *B0, *A1, *OUT; };
-struct BlkIdx { int tw, tb, c0w, c0b, g0, b0, c1w, c1b, g1, b1, rw, rb; };
 
 struct TrainState {
   int cap_rows = 0;
@@ -1023,49 +1022,28 @@ int unet_train_backward(CldHandle* h, const float* d_eps, float* const* grads, i
   const CldConfig& c = h->cfg;
   const int T = c.horizon, T2 = T / 2, T4 = T / 4;
   const int d0 = c.dims[0], d1 = c.dims[1], d2 = c.dims[2], D = c.latent_dim, td = c.base_dim, tdim = c.base_dim + c.cond_dim;
-  // ---- parameter indices in state-dict order (the order cld_load_unet consumes)
-  BlkIdx ix[12];
-  int i_down[2][2], i_up[2][2], i_fin[6];
-  {
-    const int order[12] = {0, 1, 2, 3, 4, 5, 8, 9, 10, 11, 6, 7};   // exec index of the blocks in state-dict order
-    int idx = 4, k = 0;
-    auto blk = [&](int e) {
-      BlkIdx& b = ix[e];
-      b.tw = idx++; b.tb = idx++; b.c0w = idx++; b.c0b = idx++; b.g0 = idx++; b.b0 = idx++;
-      b.c1w = idx++; b.c1b = idx++; b.g1 = idx++; b.b1 = idx++;
-      if (u.rb[e].res.w) { b.rw = idx++; b.rb = idx++; } else b.rw = b.rb = -1;
-    };
-    for (int lvl = 0; lvl < 3; ++lvl) {
-      blk(order[k++]); blk(order[k++]);
-      if (lvl < 2) { i_down[lvl][0] = idx++; i_down[lvl][1] = idx++; }
-    }
-    for (int lvl = 0; lvl < 2; ++lvl) {
-      blk(order[k++]); blk(order[k++]);
-      i_up[lvl][0] = idx++; i_up[lvl][1] = idx++;
-    }
-    blk(order[k++]); blk(order[k++]);
-    for (int i = 0; i < 6; ++i) i_fin[i] = idx++;
-    if (idx != n) return fail(h, CLD_ERR_ARG, "cld_unet_backward: expected %d gradient tensors, got %d", idx, n);
-  }
+  const UnetLayout& L = h->unet_layout;
+  if (n != (int)L.numel.size()) return fail(h, CLD_ERR_ARG, "cld_unet_backward: expected %zu gradient tensors, got %d", L.numel.size(), n);
+  const BlkIdx* ix = L.blk;
   int rc, splits;
   const BlkStash* b = st->blk;
   st->unit = 0; st->nd = 0;
   auto nb = [&]() -> float* { return st->gD[st->nd < TrainState::MAX_GD ? st->nd++ : TrainState::MAX_GD - 1]; };   // a fresh data-gradient buffer
   float *g, *g2, *gA;
   // ---- final_conv: Conv1d(1x1) <- Conv1dBlock
-  if ((rc = conv_param_grads(h, d0, D, 1, st->fB, d0, nullptr, 0, T, d_eps, grads[i_fin[4]], grads[i_fin[5]], R, s))) return rc;
+  if ((rc = conv_param_grads(h, d0, D, 1, st->fB, d0, nullptr, 0, T, d_eps, grads[L.fin[4]], grads[L.fin[5]], R, s))) return rc;
   g = nb();
   {
     const int tap0[5] = {0, 0, 0, 0, 0};
     if ((rc = conv_dgrad(h, u.fin1, 1, tap0, kOff1, d_eps, T, g, T, d0, T, 1, 1, 0, 0, R, s))) return rc;
   }
-  if ((rc = gn_bwd(h, st->fA, u.fin0n, g, &gA, grads[i_fin[2]], grads[i_fin[3]], grads[i_fin[1]], nullptr, T, d0, R, s))) return rc;
-  if ((rc = conv_param_grads(h, d0, d0, 5, st->q1, d0, nullptr, 0, T, gA, grads[i_fin[0]], nullptr, R, s))) return rc;
+  if ((rc = gn_bwd(h, st->fA, u.fin0n, g, &gA, grads[L.fin[2]], grads[L.fin[3]], grads[L.fin[1]], nullptr, T, d0, R, s))) return rc;
+  if ((rc = conv_param_grads(h, d0, d0, 5, st->q1, d0, nullptr, 0, T, gA, grads[L.fin[0]], nullptr, R, s))) return rc;
   g = nb();
   if ((rc = conv_dgrad(h, u.fin0, 5, kTap5, kNeg5, gA, T, g, T, d0, T, 1, 1, 0, 0, R, s))) return rc;               // g = d q1
   // ---- ups.1: upsample, blocks 11, 10
   g2 = nb();
-  if ((rc = up_bwd(h, u.up[1], b[11].OUT, T2, g, g2, grads[i_up[1][0]], grads[i_up[1][1]], R, s))) return rc;       // g2 = d o11
+  if ((rc = up_bwd(h, u.up[1], b[11].OUT, T2, g, g2, grads[L.up[1][0]], grads[L.up[1][1]], R, s))) return rc;       // g2 = d o11
   g = nb();
   if ((rc = block_bwd(h, 11, ix[11], g2, g, grads, R, s))) return rc;                                               // g = d o10
   if ((rc = block_bwd(h, 10, ix[10], g, st->gcat10, grads, R, s))) return rc;                                       // (d q0 | d sk1)
@@ -1073,7 +1051,7 @@ int unet_train_backward(CldHandle* h, const float* d_eps, float* const* grads, i
   if ((rc = slice(h, g, st->gcat10, (size_t)R * T2, d1, 2 * d1, 0, 0, s))) return rc;                               // g = d q0
   // ---- ups.0: upsample, blocks 9, 8
   g2 = nb();
-  if ((rc = up_bwd(h, u.up[0], b[9].OUT, T4, g, g2, grads[i_up[0][0]], grads[i_up[0][1]], R, s))) return rc;        // g2 = d o9
+  if ((rc = up_bwd(h, u.up[0], b[9].OUT, T4, g, g2, grads[L.up[0][0]], grads[L.up[0][1]], R, s))) return rc;        // g2 = d o9
   g = nb();
   if ((rc = block_bwd(h, 9, ix[9], g2, g, grads, R, s))) return rc;                                                 // g = d o8
   if ((rc = block_bwd(h, 8, ix[8], g, st->gcat8, grads, R, s))) return rc;                                          // (d o7 | d sk2)
@@ -1092,7 +1070,7 @@ int unet_train_backward(CldHandle* h, const float* d_eps, float* const* grads, i
   if ((rc = block_bwd(h, 4, ix[4], g2, g, grads, R, s))) return rc;                                                 // g = d p1
   // ---- downs.1: downsample, blocks 3, 2
   g2 = nb();
-  if ((rc = down_bwd(h, u.down[1], b[3].OUT, T2, g, g2, grads[i_down[1][0]], grads[i_down[1][1]], R, s))) return rc;    // g2 = d o3 (down part)
+  if ((rc = down_bwd(h, u.down[1], b[3].OUT, T2, g, g2, grads[L.down[1][0]], grads[L.down[1][1]], R, s))) return rc;    // g2 = d o3 (down part)
   if ((rc = slice(h, g2, st->gcat10, (size_t)R * T2, d1, 2 * d1, d1, 1, s))) return rc;                             // + skip part
   g = nb();
   if ((rc = block_bwd(h, 3, ix[3], g2, g, grads, R, s))) return rc;                                                 // g = d o2
@@ -1100,7 +1078,7 @@ int unet_train_backward(CldHandle* h, const float* d_eps, float* const* grads, i
   if ((rc = block_bwd(h, 2, ix[2], g, g2, grads, R, s))) return rc;                                                 // g2 = d p0
   // ---- downs.0: downsample, blocks 1, 0
   g = nb();
-  if ((rc = down_bwd(h, u.down[0], b[1].OUT, T, g2, g, grads[i_down[0][0]], grads[i_down[0][1]], R, s))) return rc;     // g = d o1
+  if ((rc = down_bwd(h, u.down[0], b[1].OUT, T, g2, g, grads[L.down[0][0]], grads[L.down[0][1]], R, s))) return rc;     // g = d o1
   g2 = nb();
   if ((rc = block_bwd(h, 1, ix[1], g, g2, grads, R, s))) return rc;                                                 // g2 = d o0
   g = nb();
@@ -1128,11 +1106,11 @@ int unet_train_backward(CldHandle* h, const float* d_eps, float* const* grads, i
   CLD_LAUNCH_OK(h, "time_mlp_bwd_kernel");
   // Linear(d, 4d): weight [4d][d];  Linear(4d, d): weight [d][4d]
   if ((rc = conv_wgrad(h, td, 4 * td, 1, kOff1, st->emb, td, nullptr, 0, 1, st->dpre1, 1, 1, 1, 1, 0, R, &splits, ps))) return rc;
-  if ((rc = wreduce(h, splits, 1, td, 4 * td, 0, 4 * td, grads[0], 1, kK1, 0, ps))) return rc;
-  if ((rc = colsum(h, st->dpre1, R, 4 * td, grads[1], ps))) return rc;
+  if ((rc = wreduce(h, splits, 1, td, 4 * td, 0, 4 * td, grads[L.tmlp[0]], 1, kK1, 0, ps))) return rc;
+  if ((rc = colsum(h, st->dpre1, R, 4 * td, grads[L.tmlp[1]], ps))) return rc;
   if ((rc = conv_wgrad(h, 4 * td, td, 1, kOff1, st->hid, 4 * td, nullptr, 0, 1, st->dpre2, 1, 1, 1, 1, 0, R, &splits, ps))) return rc;
-  if ((rc = wreduce(h, splits, 1, 4 * td, td, 0, td, grads[2], 1, kK1, 0, ps))) return rc;
-  if ((rc = colsum(h, st->dpre2, R, td, grads[3], ps))) return rc;
+  if ((rc = wreduce(h, splits, 1, 4 * td, td, 0, td, grads[L.tmlp[2]], 1, kK1, 0, ps))) return rc;
+  if ((rc = colsum(h, st->dpre2, R, td, grads[L.tmlp[3]], ps))) return rc;
   pg_join(h, s);                 // the gradients are complete in the caller's stream order
   return 0;
 }

@@ -133,10 +133,6 @@ struct TcState {
   float* zeros = nullptr;
   long long* prof = nullptr;
   uint8_t* skipbuf = nullptr; int skip_stride = 0; int grid = 0;
-  // weight pointers recorded by tc_pack_* until tc_finalize
-  struct Blk { int cin, cout; const float *c0w, *c0b, *g0, *b0, *c1w, *c1b, *g1, *b1, *rw, *rb; } blk[12];
-  struct Rs { int ch; const float *w, *b; } down[2], up[2];
-  const float *fw, *fb, *fg, *fbt, *f1w, *f1b;
   bool ready = false;
 };
 
@@ -862,38 +858,6 @@ __global__ void tc_copy_scale_kernel(float* __restrict__ dst, const float* __res
 
 static TcState* st_of(CldHandle* h) { return reinterpret_cast<TcState*>(h->tc); }
 
-bool tc_enabled(const CldHandle* h) {
-  const CldConfig& c = h->cfg;
-  // horizon 16..56: 8 rows per CTA; 64..112 (multiple of 8): split-time mode, 4 rows per CTA as two half-horizon lanes each
-  const bool t_ok = (c.horizon >= 16 && c.horizon <= 56) || (c.horizon >= 64 && c.horizon <= 112 && c.horizon % 8 == 0);
-  return c.precision == CLD_PREC_BF16 && c.dims[0] == 64 && c.dims[1] == 128 && c.dims[2] == 256 && t_ok && c.latent_dim == 4;
-}
-
-int tc_pack_block(CldHandle* h, int exec_idx, int cin, int cout, const float* c0w, const float* c0b, const float* g0,
-                  const float* b0, const float* c1w, const float* c1b, const float* g1, const float* b1, const float* rw,
-                  const float* rb, cudaStream_t) {
-  if (!h->tc) h->tc = new TcState();
-  st_of(h)->blk[exec_idx] = {cin, cout, c0w, c0b, g0, b0, c1w, c1b, g1, b1, rw, rb};
-  return 0;
-}
-int tc_pack_down(CldHandle* h, int lvl, int ch, const float* w, const float* b, cudaStream_t) {
-  if (!h->tc) h->tc = new TcState();
-  st_of(h)->down[lvl] = {ch, w, b};
-  return 0;
-}
-int tc_pack_up(CldHandle* h, int lvl, int ch, const float* w, const float* b, cudaStream_t) {
-  if (!h->tc) h->tc = new TcState();
-  st_of(h)->up[lvl] = {ch, w, b};
-  return 0;
-}
-int tc_pack_final(CldHandle* h, const float* fw, const float* fb, const float* fg, const float* fbt, const float* f1w,
-                  const float* f1b, cudaStream_t) {
-  if (!h->tc) h->tc = new TcState();
-  TcState* s = st_of(h);
-  s->fw = fw; s->fb = fb; s->fg = fg; s->fbt = fbt; s->f1w = f1w; s->f1b = f1b;
-  return 0;
-}
-
 namespace {
 struct Level { int T, pitch, offB, npanels, n_tiles, slot0[4], lo[4], hi[4]; };
 
@@ -955,10 +919,11 @@ TcOp blank_op() {
 }
 }  // namespace
 
-int tc_finalize(CldHandle* h, cudaStream_t stream) {
+int tc_finalize(CldHandle* h, const float* const* p, cudaStream_t stream) {
+  if (!h->tc) h->tc = new TcState();
   TcState* s = st_of(h);
-  if (!s) return fail(h, CLD_ERR_STATE, "tc_finalize without weights");
   const CldConfig& c = h->cfg;
+  const UnetLayout& sd = h->unet_layout;
   s->tsplit = c.horizon > 56;
   const int T = s->tsplit ? c.horizon / 2 : c.horizon;
   s->t_eff = T;
@@ -987,7 +952,6 @@ int tc_finalize(CldHandle* h, cudaStream_t stream) {
   }
   Builder B{s};
   s->ops.clear(); s->kbs.clear();
-  const int tb_off_exec[12] = {0, 64, 128, 256, 384, 640, 896, 1152, 1408, 1536, 1664, 1728};
   const int k5[5] = {0, 1, 2, 3, 4}, o5[5] = {-2, -1, 0, 1, 2}, k1[1] = {0}, o1[1] = {0};
   const int k3[3] = {0, 1, 2}, o3[3] = {-1, 0, 1};
   const int kue[2] = {1, 3}, oue[2] = {0, -1}, kuo[2] = {0, 2}, ouo[2] = {1, 0};
@@ -997,13 +961,14 @@ int tc_finalize(CldHandle* h, cudaStream_t stream) {
   if (const char* e = getenv("CLD_TC_SPLIT_MIN")) { int v = atoi(e); if (v == 64 || v == 128 || v == 256 || v == 512) split_min = v; }
 
   auto res_block = [&](int e, int lvl, const int* in_panels, int n_in, bool concat, int stage) {
-    const TcState::Blk& bk = s->blk[e];
+    const BlkIdx& bk = sd.blk[e];
+    const ResBlockW& rb = h->unet.rb[e];
     const Level& lv = L[lvl];
-    const int N = bk.cout, half = N / 2;
-    const bool has_res = bk.rw != nullptr;
-    const ConvSpec conv0{bk.c0w, N, bk.cin, 5, 0, k5, o5, 5, e == 0};
-    const ConvSpec resc{bk.rw, N, bk.cin, 1, 0, k1, o1, 1, e == 0};
-    const ConvSpec conv1{bk.c1w, N, N, 5, 0, k5, o5, 5, false};
+    const int N = rb.cout, half = N / 2;
+    const bool has_res = bk.rw >= 0;
+    const ConvSpec conv0{p[bk.c0w], N, rb.cin, 5, 0, k5, o5, 5, e == 0};
+    const ConvSpec resc{has_res ? p[bk.rw] : nullptr, N, rb.cin, 1, 0, k1, o1, 1, e == 0};
+    const ConvSpec conv1{p[bk.c1w], N, N, 5, 0, k5, o5, 5, false};
     // ---- op A: conv0 (+ residual 1x1 conv into the second accumulator set), GroupNorm + Mish + time bias
     // an M=128 MMA costs >= 64 cycles whatever its N (A-operand fetch), so only N = 256 layers are split into halves
     const bool csA = (N >= split_min) && !concat;    // concat blocks write h over x: the epilogue must wait for all MMAs
@@ -1012,7 +977,7 @@ int tc_finalize(CldHandle* h, cudaStream_t stream) {
     a.n = N; set_tiles(a, lv); a.kb_first = (int)s->kbs.size();
     a.epi = EPI_GN_TB; a.cout = N; a.cpg = N / 8; a.t_out = lv.T; a.n_vt = lv.n_tiles;
     a.dst_off = concat ? 0 : lv.offB; a.dst_pitch = lv.pitch;
-    a.par_off = B.add_par(bk.c0b, bk.g0, bk.b0, nullptr, N); a.tb_off = tb_off_exec[e];
+    a.par_off = B.add_par(p[bk.c0b], p[bk.g0], p[bk.b0], nullptr, N); a.tb_off = rb.tb_off;
     a.flags = (csA ? F_COMMIT_SPLIT : 0) | (skA ? F_SPLIT_K : 0);
     if (csA) {
       bool f0 = true, f1 = true, fr0 = true, fr1 = true;
@@ -1040,7 +1005,7 @@ int tc_finalize(CldHandle* h, cudaStream_t stream) {
     b.n = N; set_tiles(b, lv); b.kb_first = (int)s->kbs.size();
     b.epi = has_res ? EPI_GN_RES_ACC : EPI_GN_RES_ID; b.cout = N; b.cpg = N / 8; b.t_out = lv.T; b.n_vt = lv.n_tiles;
     b.dst_off = 0; b.dst_pitch = lv.pitch;
-    b.par_off = B.add_par(bk.c1b, bk.g1, bk.b1, bk.rb, N);
+    b.par_off = B.add_par(p[bk.c1b], p[bk.g1], p[bk.b1], has_res ? p[bk.rb] : nullptr, N);
     b.flags = (csB ? F_COMMIT_SPLIT : 0) | (skB ? F_SPLIT_K : 0);
     int hp[4];
     const int nhp = N / 64;
@@ -1093,12 +1058,12 @@ int tc_finalize(CldHandle* h, cudaStream_t stream) {
   // level 0
   panels_of(0, L[0].pitch, 1, pa); res_block(0, 0, pa, 1, false, 0);
   res_block(1, 0, pa, 1, false, 1);
-  resample(false, 64, s->down[0].w, s->down[0].b, L[0], L[1], pa, 1, 2);
+  resample(false, 64, p[sd.down[0][0]], p[sd.down[0][1]], L[0], L[1], pa, 1, 2);
   // level 1
   panels_of(0, L[1].pitch, 1, pa); res_block(2, 1, pa, 1, false, 3);
   panels_of(0, L[1].pitch, 2, pa); res_block(3, 1, pa, 2, false, 4);
   s->ops.back().save_skip = skip1_off;
-  resample(false, 128, s->down[1].w, s->down[1].b, L[1], L[2], pa, 2, 5);
+  resample(false, 128, p[sd.down[1][0]], p[sd.down[1][1]], L[1], L[2], pa, 2, 5);
   // level 2
   panels_of(0, L[2].pitch, 2, pa); res_block(4, 2, pa, 2, false, 6);
   panels_of(0, L[2].pitch, 4, pa); res_block(5, 2, pa, 4, false, 7);
@@ -1114,30 +1079,30 @@ int tc_finalize(CldHandle* h, cudaStream_t stream) {
   res_block(8, 2, pa, 8, true, 10);
   panels_of(0, L[2].pitch, 2, pa); res_block(9, 2, pa, 2, false, 11);
   {  // ups.0.2: transposed conv 128 -> 128, level 2 -> level 1 (two output phases); then skip1 into region B
-    TcOp& u = resample(true, 128, s->up[0].w, s->up[0].b, L[2], L[1], pa, 2, 12);
+    TcOp& u = resample(true, 128, p[sd.up[0][0]], p[sd.up[0][1]], L[2], L[1], pa, 2, 12);
     u.load_skip = skip1_off; u.load_off = L[1].offB; u.load_pitch = L[1].pitch; u.load_npanels = 2; u.load_T = L[1].T;
   }
   // level 1 (up path)
   panels_of(0, L[1].pitch, 2, pa); panels_of(L[1].offB, L[1].pitch, 2, pa + 2);
   res_block(10, 1, pa, 4, true, 13);
   panels_of(0, L[1].pitch, 1, pa); res_block(11, 1, pa, 1, false, 14);
-  resample(true, 64, s->up[1].w, s->up[1].b, L[1], L[0], pa, 1, 15);
+  resample(true, 64, p[sd.up[1][0]], p[sd.up[1][1]], L[1], L[0], pa, 1, 15);
   {  // final_conv.0: conv k5 + GroupNorm + Mish -> region B ; final_conv.1: 1x1 conv 64 -> 4 -> eps
     panels_of(0, L[0].pitch, 1, pa);
     TcOp f = blank_op();
     f.n = 64; set_tiles(f, L[0]); f.kb_first = (int)s->kbs.size();
     f.epi = EPI_GN; f.cout = 64; f.cpg = 8; f.t_out = L[0].T; f.n_vt = L[0].n_tiles; f.dst_off = L[0].offB; f.dst_pitch = L[0].pitch;
-    f.par_off = B.add_par(s->fb, s->fg, s->fbt, nullptr, 64); f.dbg_stage = 16;
-    const ConvSpec cf{s->fw, 64, 64, 5, 0, k5, o5, 5, false};
+    f.par_off = B.add_par(p[sd.fin[1]], p[sd.fin[2]], p[sd.fin[3]], nullptr, 64); f.dbg_stage = 16;
+    const ConvSpec cf{p[sd.fin[0]], 64, 64, 5, 0, k5, o5, 5, false};
     bool ff = true;
     f.n_g0 = B.emit(cf, pa, 0, 1, 0, 64, 0, ff);
     s->ops.push_back(f);
     TcOp g = blank_op();
     g.n = 16; set_tiles(g, L[0]); g.kb_first = (int)s->kbs.size();
     g.epi = EPI_OUT; g.cout = 4; g.t_out = L[0].T; g.n_vt = L[0].n_tiles;
-    g.par_off = B.add_par(s->f1b, nullptr, nullptr, nullptr, 4);
+    g.par_off = B.add_par(p[sd.fin[5]], nullptr, nullptr, nullptr, 4);
     panels_of(L[0].offB, L[0].pitch, 1, pa);
-    const ConvSpec cg{s->f1w, 4, 64, 1, 0, k1, o1, 1, false};
+    const ConvSpec cg{p[sd.fin[4]], 4, 64, 1, 0, k1, o1, 1, false};
     bool fg = true;
     g.n_g0 = B.emit(cg, pa, 0, 1, 0, 16, 0, fg);
     s->ops.push_back(g);

@@ -3,15 +3,8 @@
 #include "common.cuh"
 
 namespace cld {
-bool tc_enabled(const CldHandle* h);
-int tc_pack_block(CldHandle* h, int exec_idx, int cin, int cout, const float* c0w, const float* c0b, const float* g0,
-                  const float* b0, const float* c1w, const float* c1b, const float* g1, const float* b1,
-                  const float* rw, const float* rb, cudaStream_t s);
-int tc_pack_down(CldHandle* h, int lvl, int ch, const float* w, const float* b, cudaStream_t s);
-int tc_pack_up(CldHandle* h, int lvl, int ch, const float* w, const float* b, cudaStream_t s);
-int tc_pack_final(CldHandle* h, const float* fw, const float* fb, const float* fg, const float* fbt, const float* f1w,
-                  const float* f1b, cudaStream_t s);
-int tc_finalize(CldHandle* h, cudaStream_t s);
+// packs the bf16 weight images from the state-dict tensors `p` (indices of h->unet_layout)
+int tc_finalize(CldHandle* h, const float* const* p, cudaStream_t s);
 int tc_unet_forward(CldHandle* h, const float* x, const float* cond, const int64_t* t, float* eps, int R,
                     cudaStream_t s);
 // same, with h->tbias (cond part) and h->tvec (time part) already computed by unet_cond_bias / unet_time_vec

@@ -122,7 +122,9 @@ const char* cld_last_error(const CldHandle* h);   /* h may be NULL: last create(
 
 /* Denoiser weights: the 148 tensors of DmModel.model.state_dict() in state-dict order
  * (SURVEY.md sec. 8b), fp32 device pointers; numels[i] (optional, may be NULL) is checked against
- * the element count the layout expects.  Packs them into the kernels' layouts.
+ * the element count the layout expects.  Packs them into the kernels' layouts.  On an fp32 handle every call, the first
+ * included, is ONE kernel launch with no allocation and no synchronise, so it may be captured in a CUDA graph.  An argument
+ * error is reported before anything is written: the loaded weights are unchanged.
  * Replaces: TemporalMapUnet.__init__/load_state_dict (src/tbsim/models/temporal.py:49-120). */
 int cld_load_unet(CldHandle* h, const float* const* dev_ptrs, const int64_t* numels, int n, void* stream);
 
