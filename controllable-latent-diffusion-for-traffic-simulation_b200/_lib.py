@@ -42,6 +42,7 @@ class CldGuidanceConfig(C.Structure):
         ("min_target_time", C.c_float), ("optimizer", C.c_int32), ("lr", C.c_float),
         ("w_target_speed", C.c_float), ("w_acc_limit", C.c_float), ("acc_limit", C.c_float),
         ("w_speed_limit", C.c_float), ("speed_limit", C.c_float), ("w_waypoint", C.c_float),
+        ("grad_steps", C.c_int32),
     ]
 
 

@@ -532,7 +532,19 @@ int cld_indicators(CldHandle* h, const float* traj, const CldScene* scene, uint8
   return indicators(h, traj, scene, offroad_out, coll_out, reward_out, R, (cudaStream_t)stream);
 }
 
-// h0 == nullptr: compute cond2hidden(cond) first; otherwise cond is unused
+// checks CldGuidanceConfig.grad_steps and, for a multi-step Adam call, allocates the moment buffers on first use
+static int guidance_prepare_steps(CldHandle* h, const CldGuidanceConfig* g) {
+  if (g->grad_steps < 0) return fail(h, CLD_ERR_ARG, "grad_steps must be >= 0 (0 and 1 both mean one iteration), got %d", g->grad_steps);
+  if (g->grad_steps <= 1 || g->optimizer != CLD_OPT_ADAM) return 0;
+  const size_t n = (size_t)h->cfg.max_rows * h->cfg.horizon * 4;
+  int rc;
+  if ((rc = dev_alloc(h, &h->ws_adam_m, n))) return rc;
+  return dev_alloc(h, &h->ws_adam_v, n);
+}
+
+// h0 == nullptr: compute cond2hidden(cond) first; otherwise cond is unused.  g->grad_steps iterations of decode (with stash) ->
+// losses -> BPTT + optimizer step: iteration 1 reads z_mean, later ones the z_out of the one before (in place: each row reads
+// its z before it writes it); grad_out / loss_out keep the last iteration's values.
 static int guidance_step_impl(CldHandle* h, const float* z_mean, const float* cond, const float* h0, const float* curr,
                               const CldScene* scene, const CldGuidanceConfig* g, float* z_out, float* grad_out,
                               float* loss_out, int R, cudaStream_t s) {
@@ -541,13 +553,30 @@ static int guidance_step_impl(CldHandle* h, const float* z_mean, const float* co
     if ((rc = decode_h0(h, cond, h->ws_h0, R, s))) return rc;
     h0 = h->ws_h0;
   }
-  if ((rc = decode_rollout_h0(h, z_mean, h0, curr, h->ws_act, h->ws_traj, true, R, s))) return rc;
   // bf16 mode without per-row loss output (the sampler): the two loss kernels run concurrently, each into its own buffer
   float* dmap = (h->use_lstm_tc && !loss_out && g->w_map_collision != 0.f && !h->env_lstm_bwd_simt &&
                  !h->env_guidance_nofork) ? h->ws_dtraj2 : nullptr;
   float* dacc = g->w_acc_limit != 0.f ? h->ws_dacc : nullptr;
-  if ((rc = guidance_loss_grad(h, h->ws_traj, scene, g, h->ws_dtraj, dmap, dacc, loss_out, R, s))) return rc;
-  return decode_backward_update2(h, z_mean, h->ws_act, curr, h->ws_dtraj, dmap, dacc, g, z_out, grad_out, R, s);
+  const int steps = g->grad_steps > 1 ? g->grad_steps : 1;
+  const bool moments = steps > 1 && g->optimizer == CLD_OPT_ADAM;
+  if (moments && !h->ws_adam_m) return fail(h, CLD_ERR_STATE, "internal: Adam moment buffers not allocated");
+  for (int it = 1; it <= steps; ++it) {
+    const float* z = it == 1 ? z_mean : z_out;
+    const bool last = it == steps;
+    GuideOpt opt;
+    opt.iter = it;
+    if (moments) {
+      // torch.optim.Adam derives its scalar factors in double: step_size = lr / bc1, bc2 ** 0.5
+      opt.m = h->ws_adam_m; opt.v = h->ws_adam_v;
+      opt.step_size = (float)((double)g->lr / (1.0 - pow(0.9, it)));
+      opt.bc2_sqrt = (float)sqrt(1.0 - pow(0.999, it));
+    }
+    if ((rc = decode_rollout_h0(h, z, h0, curr, h->ws_act, h->ws_traj, true, R, s))) return rc;
+    if ((rc = guidance_loss_grad(h, h->ws_traj, scene, g, h->ws_dtraj, dmap, dacc, last ? loss_out : nullptr, R, s))) return rc;
+    if ((rc = decode_backward_update2(h, z, h->ws_act, curr, h->ws_dtraj, dmap, dacc, g, opt, z_out, last ? grad_out : nullptr, R, s)))
+      return rc;
+  }
+  return 0;
 }
 
 int cld_guidance_step(CldHandle* h, const float* z_mean, const float* cond, const float* curr, const CldScene* scene,
@@ -555,6 +584,7 @@ int cld_guidance_step(CldHandle* h, const float* z_mean, const float* cond, cons
   int rc = check_rows(h, R);
   if (rc) return rc;
   if (!z_mean || !cond || !curr || !scene || !g || !z_out) return fail(h, CLD_ERR_ARG, "null argument");
+  if ((rc = guidance_prepare_steps(h, g))) return rc;
   if (g->w_map_collision != 0.f && (rc = guidance_prepare_maps(h, scene, (cudaStream_t)stream))) return rc;
   return guidance_step_impl(h, z_mean, cond, nullptr, curr, scene, g, z_out, grad_out, loss_out, R, (cudaStream_t)stream);
 }
@@ -570,6 +600,8 @@ int cld_sample(CldHandle* h, const float* x_init, const float* noises, uint64_t 
   if ((traj_out || offroad_out || coll_out || g) && !curr) return fail(h, CLD_ERR_ARG, "curr states required");
   if ((offroad_out || coll_out || g) && !scene) return fail(h, CLD_ERR_ARG, "scene tensors required");
   if (!h->sched.loaded) return fail(h, CLD_ERR_STATE, "schedule not set");
+  int rc;
+  if (g && (rc = guidance_prepare_steps(h, g))) return rc;
   cudaStream_t s = (cudaStream_t)stream;
   const CldConfig& c = h->cfg;
   const int T = c.horizon, D = c.latent_dim, n_t = c.n_timesteps;
@@ -587,7 +619,6 @@ int cld_sample(CldHandle* h, const float* x_init, const float* noises, uint64_t 
   }
   int chunk = (c.max_rows / unit) * unit;
   if (chunk < unit) return fail(h, CLD_ERR_ARG, "max_rows=%d is smaller than one scene (A*N=%d)", c.max_rows, unit);
-  int rc;
   for (int r0 = 0; r0 < R; r0 += chunk) {
     const int Rc = (R - r0 < chunk) ? (R - r0) : chunk;
     CldScene sub;

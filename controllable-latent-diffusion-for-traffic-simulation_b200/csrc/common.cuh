@@ -124,6 +124,9 @@ struct CldHandle {
   float* ws_dtraj = nullptr;       // [max_rows, T, 4]
   float* ws_dtraj2 = nullptr;      // [max_rows, T, 4] map-collision part when it runs concurrently (bf16 mode sampler)
   float* ws_dacc = nullptr;        // [max_rows, T] d/d(acc) of the acc-limit guidance term
+  // Adam moments (m, v) of a guided step with grad_steps > 1, [max_rows, T, 4] each: allocated on first use
+  float* ws_adam_m = nullptr;
+  float* ws_adam_v = nullptr;
   // map-collision guidance: work list of the (row, step) items whose footprint may cross a road edge (+ 2 counters), and the
   // one-bit-per-pixel copy of byte-per-pixel drivable maps that the screen reads (guidance_prepare_maps; bit-packed scenes are read in place)
   int* map_work = nullptr;
@@ -246,16 +249,28 @@ int fill_t(CldHandle* h, int64_t* t, int value, int R, cudaStream_t s);
 int decode_rollout(CldHandle* h, const float* z, const float* cond, const float* curr, float* act_out,
                    float* traj_out, bool save, int R, cudaStream_t s);
 int unicycle(CldHandle* h, const float* curr, const float* u, float* state_out, int R, cudaStream_t s);
+// optimizer iteration `iter` (1-based) of a guided step.  m == nullptr: the single-iteration update (torch's first Adam step, or
+// SGD), no moment traffic.  Otherwise Adam with moments m / v [R,T,4]: iteration 1 writes m = 0.1 g, v = 0.001 g^2 next to the
+// first-step update, iteration >= 2 reads and updates them and steps z -= step_size * m / (sqrt(v) / bc2_sqrt + 1e-8).
+struct GuideOpt {
+  int iter = 1;
+  float* m = nullptr;
+  float* v = nullptr;
+  float step_size = 0.f;     // lr / (1 - 0.9^iter)
+  float bc2_sqrt = 0.f;      // sqrt(1 - 0.999^iter)
+};
 // ---- kernels_lstm.cu
 int decode_h0(CldHandle* h, const float* cond, float* h0, int R, cudaStream_t s);
 int decode_backward_update2(CldHandle* h, const float* z_mean, const float* act, const float* curr, const float* dtraj,
-                            const float* dtraj2, const float* dacc, const CldGuidanceConfig* g, float* z_out, float* grad_out, int R, cudaStream_t s);
+                            const float* dtraj2, const float* dacc, const CldGuidanceConfig* g, const GuideOpt& opt, float* z_out,
+                            float* grad_out, int R, cudaStream_t s);
 int decode_rollout_h0(CldHandle* h, const float* z, const float* h0, const float* curr, float* act_out, float* traj_out,
                       bool save, int R, cudaStream_t s);
 int decode_rollout_h0_tc(CldHandle* h, const float* z, const float* h0, const float* curr, float* act_out, float* traj_out,
                          bool save, int R, cudaStream_t s);
 int decode_backward_update_tc(CldHandle* h, const float* z_mean, const float* act, const float* curr, const float* dtraj,
-                              const float* dtraj2, const float* dacc, const CldGuidanceConfig* g, float* z_out, float* grad_out, int R, cudaStream_t s);
+                              const float* dtraj2, const float* dacc, const CldGuidanceConfig* g, const GuideOpt& opt, float* z_out,
+                              float* grad_out, int R, cudaStream_t s);
 void lstm_tc_destroy(CldHandle* h);
 int indicators(CldHandle* h, const float* traj, const CldScene* sc, uint8_t* offroad, float* coll,
                float* reward, int R, cudaStream_t s);

@@ -265,7 +265,7 @@ __global__ void __launch_bounds__(LS_THREADS, 1) lstm_decode2_kernel(const Lstm2
 }
 
 // ------------------------------------------------------------------------------------------------
-// backward: d(traj) -> d(scaled actions) -> BPTT through both layers -> dz -> first optimizer step
+// backward: d(traj) -> d(scaled actions) -> BPTT through both layers -> dz -> optimizer step
 // (PerturbationGuidance.perturb, reference src/tbsim/utils/guidance_loss.py:2250-2278).  Same tiling as the
 // forward: one CTA owns 32 rows; pass 1 walks layer 1 backwards in time with [W_hh1 | W_ih1]^T in shared memory
 // (per step: gate gradients [32 x 256] x [256 x 128] -> recurrent dh1 (kept in registers by the thread that needs it
@@ -287,6 +287,7 @@ struct Bwd2Args {
   int R, T;
   DynParams2 dyn;
   int optimizer; float lr;
+  GuideOpt opt;                         // iteration and Adam moments of a multi-step guided call
 };
 
 // packs W_hh [256][64] | W_ih [256][in] (nn.LSTM layouts) into [j pair][col][2], col < 64: W_hh[j][col], else W_ih[j][col-64]
@@ -500,12 +501,19 @@ __global__ void __launch_bounds__(LS_THREADS, 1) lstm_backward2_kernel(const Bwd
       const float g = dzs[i], z = a.z_mean[gi_];
       float zn;
       if (a.optimizer == CLD_OPT_ADAM) {
-        // first torch.optim.Adam step: m = 0.1 g, v = 0.001 g^2, bias corrections 0.1 / 0.001, eps 1e-8
-        const float m = 0.1f * g;
-        const float v = (0.001f * g) * g;
-        const float denom = sqrtf(v) / 0.03162277660168379f + 1e-8f;
-        const float step = a.lr / 0.1f;
-        zn = z - step * (m / denom);
+        float m, v;
+        if (!a.opt.m) {
+          zn = adam_first_step(z, g, a.lr, m, v);
+        } else {
+          // multi-step call: the moments live across iterations
+          if (a.opt.iter == 1) {
+            zn = adam_first_step(z, g, a.lr, m, v);
+          } else {
+            m = a.opt.m[gi_]; v = a.opt.v[gi_];
+            zn = adam_next_step(z, g, a.opt.step_size, a.opt.bc2_sqrt, m, v);
+          }
+          a.opt.m[gi_] = m; a.opt.v[gi_] = v;
+        }
       } else {
         zn = z - a.lr * g;
       }
@@ -577,10 +585,12 @@ int decode_rollout_h0(CldHandle* h, const float* z, const float* h0, const float
 
 
 int decode_backward_update2(CldHandle* h, const float* z_mean, const float* act, const float* curr, const float* dtraj,
-                            const float* dtraj2, const float* dacc, const CldGuidanceConfig* g, float* z_out, float* grad_out, int R, cudaStream_t s) {
+                            const float* dtraj2, const float* dacc, const CldGuidanceConfig* g, const GuideOpt& opt, float* z_out,
+                            float* grad_out, int R, cudaStream_t s) {
   DecoderW& w = h->dec;
   int rc;
-  if (h->use_lstm_tc && !h->env_lstm_bwd_simt) return decode_backward_update_tc(h, z_mean, act, curr, dtraj, dtraj2, dacc, g, z_out, grad_out, R, s);
+  if (h->use_lstm_tc && !h->env_lstm_bwd_simt)
+    return decode_backward_update_tc(h, z_mean, act, curr, dtraj, dtraj2, dacc, g, opt, z_out, grad_out, R, s);
   if (dtraj2) return fail(h, CLD_ERR_STATE, "internal: split d(traj) buffers are only handled by the tensor-core backward");
   if ((rc = lstm2_prepare(h, s))) return rc;
   const CldConfig& c = h->cfg;
@@ -592,7 +602,7 @@ int decode_backward_update2(CldHandle* h, const float* z_mean, const float* act,
   a.dyn.dt = c.dt; a.dyn.acce_lo = c.acce_lo; a.dyn.acce_hi = c.acce_hi; a.dyn.v_lo = c.v_lo; a.dyn.v_hi = c.v_hi;
   a.dyn.max_steer = c.max_steer; a.dyn.max_yawvel = c.max_yawvel;
   a.dyn.a_mean = c.norm_mean[4]; a.dyn.a_std = c.norm_std[4]; a.dyn.w_mean = c.norm_mean[5]; a.dyn.w_std = c.norm_std[5];
-  a.optimizer = g->optimizer; a.lr = g->lr;
+  a.optimizer = g->optimizer; a.lr = g->lr; a.opt = opt;
   lstm_backward2_kernel<<<(R + LS_RB - 1) / LS_RB, LS_THREADS, lb_smem(a.T), s>>>(a);
   CLD_LAUNCH_OK(h, "lstm_backward2_kernel");
   return 0;

@@ -505,6 +505,7 @@ struct BwdTcArgs {
   int R, T;
   DynParams2 dyn;
   int optimizer; float lr;
+  GuideOpt opt;                         // iteration and Adam moments of a multi-step guided call
   int pf;                               // L2 prefetch distance in steps (0: off)
 };
 
@@ -543,7 +544,9 @@ __device__ __forceinline__ void ld8(const float* p, float (&o)[8]) {
                : "=f"(o[0]), "=f"(o[1]), "=f"(o[2]), "=f"(o[3]), "=f"(o[4]), "=f"(o[5]), "=f"(o[6]), "=f"(o[7]) : "l"(p) : "memory");
 }
 
-template <bool PROF>
+// MOM: the Adam moments of a multi-step guided call (a.opt.m, a.opt.v) are read / written; the single-iteration instance has no
+// moment code at all
+template <bool PROF, bool MOM>
 __global__ void __launch_bounds__(LB_THREADS, 1) lstm_backward_tc_kernel(const BwdTcArgs a) {
   constexpr int P0 = 20, PN = 4;        // CLD_LSTM_PROF=1: timeline of steps P0 .. P0+PN-1 of CTA 0 (clock64), printed at the end
   long long tl[PN][4];
@@ -806,23 +809,29 @@ __global__ void __launch_bounds__(LB_THREADS, 1) lstm_backward_tc_kernel(const B
                tl[k][1] - tbase, tl[k][2] - tbase, tl[k][3] - tbase);
   }
   else {
-    // ===================== warp 17: dz -> first optimizer step on z (guidance_loss.py:2250-2278), lane = row =====================
+    // ===================== warp 17: dz -> optimizer step on z (guidance_loss.py:2250-2278), lane = row =====================
     const int row = row0 + lane;
     const bool valid = row < R;
     const float is = inv_scale[lane], lr = a.lr;
     const bool adam = a.optimizer == CLD_OPT_ADAM;
+    // Adam moments of a multi-step call: iteration 1 writes them, later iterations read them back (the moments see the
+    // unscaled gradient, as grad_out does)
+    const bool mom = MOM && adam, mom_in = mom && a.opt.iter > 1;
     auto upd = [&](float z, float g) {
-      if (adam) {
-        // first torch.optim.Adam step: m = 0.1 g, v = 0.001 g^2, bias corrections 0.1 / 0.001, eps 1e-8
-        const float m = 0.1f * g;
-        const float vv = (0.001f * g) * g;
-        const float denom = sqrtf(vv) / 0.03162277660168379f + 1e-8f;
-        return z - (lr / 0.1f) * (m / denom);
-      }
+      float m, vv;
+      if (adam) return adam_first_step(z, g, lr, m, vv);
       return z - lr * g;
     };
-    float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (valid) z = reinterpret_cast<const float4*>(a.z_mean)[(size_t)row * T + (T - 1)];
+    auto upd_m = [&](float z, float g, float& m, float& vv) {
+      if (mom_in) return adam_next_step(z, g, a.opt.step_size, a.opt.bc2_sqrt, m, vv);
+      return adam_first_step(z, g, lr, m, vv);
+    };
+    const float4* zin = reinterpret_cast<const float4*>(a.z_mean);
+    float4* mp = reinterpret_cast<float4*>(a.opt.m);
+    float4* vp = reinterpret_cast<float4*>(a.opt.v);
+    float4 z = make_float4(0.f, 0.f, 0.f, 0.f), m4 = z, v4 = z;
+    if (valid) z = zin[(size_t)row * T + (T - 1)];
+    if (valid && mom_in) { m4 = mp[(size_t)row * T + (T - 1)]; v4 = vp[(size_t)row * T + (T - 1)]; }
     for (int i = 1; i <= T; ++i) {
       const int tz = T - i;
       lt_wait(bar_dz, (uint32_t)(i - 1) & 1u, 50000 + i);
@@ -831,10 +840,23 @@ __global__ void __launch_bounds__(LB_THREADS, 1) lstm_backward_tc_kernel(const B
       if (lane == 0) mbar_arrive(bar_dzfree);
       g.x *= is; g.y *= is; g.z *= is; g.w *= is;
       const float4 zc = z;
-      if (valid && tz >= 1) z = reinterpret_cast<const float4*>(a.z_mean)[(size_t)row * T + tz - 1];   // next step's z, in flight during this step
+      float4 mn = m4, vn = v4;
+      if (valid && tz >= 1) {
+        z = zin[(size_t)row * T + tz - 1];                  // next step's z (and moments), in flight during this step
+        if (mom_in) { m4 = mp[(size_t)row * T + tz - 1]; v4 = vp[(size_t)row * T + tz - 1]; }
+      }
       if (valid) {
-        reinterpret_cast<float4*>(a.z_out)[(size_t)row * T + tz] = make_float4(upd(zc.x, g.x), upd(zc.y, g.y), upd(zc.z, g.z), upd(zc.w, g.w));
-        if (a.grad_out) reinterpret_cast<float4*>(a.grad_out)[(size_t)row * T + tz] = g;
+        const size_t o = (size_t)row * T + tz;
+        if (!mom) {
+          reinterpret_cast<float4*>(a.z_out)[o] = make_float4(upd(zc.x, g.x), upd(zc.y, g.y), upd(zc.z, g.z), upd(zc.w, g.w));
+        } else {
+          float4 zn;
+          zn.x = upd_m(zc.x, g.x, mn.x, vn.x); zn.y = upd_m(zc.y, g.y, mn.y, vn.y);
+          zn.z = upd_m(zc.z, g.z, mn.z, vn.z); zn.w = upd_m(zc.w, g.w, mn.w, vn.w);
+          reinterpret_cast<float4*>(a.z_out)[o] = zn;
+          mp[o] = mn; vp[o] = vn;
+        }
+        if (a.grad_out) reinterpret_cast<float4*>(a.grad_out)[o] = g;
       }
     }
   }
@@ -870,8 +892,9 @@ static int lstm_tc_prepare(CldHandle* h, cudaStream_t s) {
   lstm_tc_pack_bwd_kernel<<<(LB_WCOLS * 128 + 255) / 256, 256, 0, s>>>(reinterpret_cast<uint32_t*>(st->wbwd), w.wih0_raw, w.whh0_raw, w.wih1_raw, w.whh1_raw);
   CLD_LAUNCH_OK(h, "lstm_tc_pack_bwd_kernel");
   if (lbk_smem(h->cfg.horizon) + 1024 > 232448) return fail(h, CLD_ERR_UNSUPPORTED, "horizon too long for the tensor-core LSTM backward");
-  CLD_CUDA_OK(h, cudaFuncSetAttribute(lstm_backward_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb_smem_req(h->cfg.horizon)));
-  CLD_CUDA_OK(h, cudaFuncSetAttribute(lstm_backward_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb_smem_req(h->cfg.horizon)));
+  CLD_CUDA_OK(h, cudaFuncSetAttribute(lstm_backward_tc_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb_smem_req(h->cfg.horizon)));
+  CLD_CUDA_OK(h, cudaFuncSetAttribute(lstm_backward_tc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb_smem_req(h->cfg.horizon)));
+  CLD_CUDA_OK(h, cudaFuncSetAttribute(lstm_backward_tc_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb_smem_req(h->cfg.horizon)));
   h->lstm_tc = st;
   return 0;
 }
@@ -902,17 +925,20 @@ int decode_rollout_h0_tc(CldHandle* h, const float* z, const float* h0, const fl
 
 
 int decode_backward_update_tc(CldHandle* h, const float* z_mean, const float* act, const float* curr, const float* dtraj,
-                              const float* dtraj2, const float* dacc, const CldGuidanceConfig* g, float* z_out, float* grad_out, int R, cudaStream_t s) {
+                              const float* dtraj2, const float* dacc, const CldGuidanceConfig* g, const GuideOpt& opt, float* z_out,
+                              float* grad_out, int R, cudaStream_t s) {
   int rc;
   if ((rc = lstm_tc_prepare(h, s))) return rc;
   const LstmTcState* st = reinterpret_cast<const LstmTcState*>(h->lstm_tc);
   BwdTcArgs a;
   a.z_mean = z_mean; a.act = act; a.curr = curr; a.dtraj = dtraj; a.dtraj2 = dtraj2; a.dacc = dacc; a.stash = h->stash; a.wblob = st->wbwd;
   a.h2a_w = h->dec.h2a_w; a.z_out = z_out; a.grad_out = grad_out; a.R = R; a.T = h->cfg.horizon; a.dyn = make_dyn2(h->cfg);
-  a.optimizer = g->optimizer; a.lr = g->lr;
+  a.optimizer = g->optimizer; a.lr = g->lr; a.opt = opt;
   a.pf = h->env_lstm_pf;
-  if (h->env_lstm_prof) lstm_backward_tc_kernel<true><<<(R + LT_RB - 1) / LT_RB, LB_THREADS, lb_smem_req(a.T), s>>>(a);
-  else lstm_backward_tc_kernel<false><<<(R + LT_RB - 1) / LT_RB, LB_THREADS, lb_smem_req(a.T), s>>>(a);
+  const int grid = (R + LT_RB - 1) / LT_RB;
+  if (opt.m) lstm_backward_tc_kernel<false, true><<<grid, LB_THREADS, lb_smem_req(a.T), s>>>(a);
+  else if (h->env_lstm_prof) lstm_backward_tc_kernel<true, false><<<grid, LB_THREADS, lb_smem_req(a.T), s>>>(a);
+  else lstm_backward_tc_kernel<false, false><<<grid, LB_THREADS, lb_smem_req(a.T), s>>>(a);
   CLD_LAUNCH_OK(h, "lstm_backward_tc_kernel");
   return 0;
 }

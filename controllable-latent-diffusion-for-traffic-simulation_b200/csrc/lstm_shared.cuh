@@ -88,4 +88,20 @@ __device__ inline void unicycle_row_backward2(const float* act, const float* cur
   }
 }
 
+// torch.optim.Adam (betas 0.9 / 0.999, eps 1e-8) on one element of z (guidance_loss.py:2250-2278).  First step, from zero
+// moments: m = 0.1 g, v = 0.001 g^2, bias corrections 0.1 / 0.001, so the update is z - lr g / (|g| + 1e-8).
+__device__ __forceinline__ float adam_first_step(float z, float g, float lr, float& m, float& v) {
+  m = 0.1f * g;
+  v = (0.001f * g) * g;
+  const float denom = sqrtf(v) / 0.03162277660168379f + 1e-8f;
+  return z - (lr / 0.1f) * (m / denom);
+}
+// a later step (torch's single-tensor form): m.lerp_(g, 0.1), v = 0.999 v + 0.001 g^2, z -= step_size m / (sqrt(v) / bc2_sqrt + eps)
+__device__ __forceinline__ float adam_next_step(float z, float g, float step_size, float bc2_sqrt, float& m, float& v) {
+  m = m + 0.1f * (g - m);
+  v = v * 0.999f + (0.001f * g) * g;
+  const float denom = sqrtf(v) / bc2_sqrt + 1e-8f;
+  return z - step_size * (m / denom);
+}
+
 }  // namespace cld

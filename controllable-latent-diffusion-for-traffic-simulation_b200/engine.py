@@ -30,6 +30,14 @@ def _u8(t, dev):
     return t.to(torch.uint8).contiguous()
 
 
+def _grad_steps(v):
+    """The guidance dict's `grad_steps`: an integer >= 1 (a bool or a float is refused rather than rounded)."""
+    import numbers
+    if isinstance(v, bool) or not isinstance(v, numbers.Integral) or int(v) < 1:
+        raise ValueError("guidance grad_steps must be an integer >= 1, got %r" % (v,))
+    return int(v)
+
+
 def _on_device(fn):
     """Run a method with the engine's device current: the handle's buffers, the kernels and the caller's stream all
     belong to `self.device`, whatever device the calling thread had selected."""
@@ -198,6 +206,7 @@ class Engine:
         gc.w_acc_limit, gc.acc_limit = float(g.get("acc_limit", 0.0)), float(g.get("acc_limit_value", 0.0))
         gc.w_speed_limit, gc.speed_limit = float(g.get("speed_limit", 0.0)), float(g.get("speed_limit_value", 0.0))
         gc.w_waypoint = float(g.get("waypoint", 0.0))
+        gc.grad_steps = _grad_steps(g.get("grad_steps", 1))
         return gc
 
     # ------------------------------------------------------------------ kernels

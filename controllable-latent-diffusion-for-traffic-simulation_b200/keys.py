@@ -19,7 +19,9 @@ def default_guidance(**over):
              # SURVEY.md sec. 8 f-4 (off by default): weights and limits of TargetSpeedLoss / AccLimitLoss / SpeedLimitLoss
              target_speed=0.0, acc_limit=0.0, acc_limit_value=0.0, speed_limit=0.0, speed_limit_value=0.0,
              # waypoint terms (cld_b200.waypoints: target_pos_at_time / global_target_pos_at_time / global_target_pos)
-             waypoint=0.0)
+             waypoint=0.0,
+             # optimizer iterations per guided denoising step (PerturbationGuidance.perturb's grad_steps)
+             grad_steps=1)
     g.update(over)
     return g
 

@@ -57,7 +57,9 @@ class GuidedDiffusionPolicy:
         act_idx = torch.zeros(B, dtype=torch.long, device=traj.device)
         losses = {}
         if self.guidance is not None:
+            # the samples are scored by ONE loss evaluation at their x0: more optimizer iterations would score a perturbed latent
             g = dict(default_guidance(), **self.guidance)
+            g["grad_steps"] = 1
             eng = self.dm.engine(B * N)
             scene = eng.make_scene(obs_dict, B // A, A, N)
             rep = (lambda v: v.repeat_interleave(N, dim=0)) if N > 1 else (lambda v: v)

@@ -85,6 +85,7 @@ typedef struct {
   float speed_limit;
   float w_waypoint;         /* waypoint terms selected per agent by CldScene.wp_mode (TargetPosAtTimeLoss guidance_loss.py:630-670; the
                                branches of GlobalTargetPosAtTimeLoss :930-1031 / GlobalTargetPosLoss :1033-1135, compute_progress_loss :876-927) */
+  int32_t grad_steps;       /* optimizer iterations per guided step (perturb's grad_steps); 0 and 1 both mean one, < 0 is CLD_ERR_ARG */
 } CldGuidanceConfig;
 
 /* Per-agent scene tensors (the reference's data_batch entries), B = S*A agent rows, scene-major. */
@@ -227,11 +228,15 @@ int cld_unicycle(CldHandle* h, const float* curr, const float* u, float* state_o
 int cld_indicators(CldHandle* h, const float* traj, const CldScene* scene, uint8_t* offroad_out,
                    float* coll_out, float* reward_out, int R, void* stream);
 
-/* One guidance update of PerturbationGuidance.perturb (guidance_loss.py:2221-2282) with
- * decoder = lstm_dec and transform = convert_action_to_state_and_action, one scene per reference
- * call: z_out = z_mean - lr*g/(|g|+1e-8) (Adam step 1) or z_mean - lr*g (SGD), g = dL/dz by an
- * analytic backward.  cond/curr are per ROW ([R,C], [R,4]).  grad_out [R,T,4] and
- * loss_out [7,R] (agent_collision, map_collision, target_pos, target_speed, acc_limit, speed_limit, waypoint per row) may be NULL. */
+/* PerturbationGuidance.perturb (guidance_loss.py:2221-2282) with decoder = lstm_dec and
+ * transform = convert_action_to_state_and_action, one scene per reference call: g->grad_steps
+ * iterations of  g = dL/dz (analytic backward), then one step of a fresh torch.optim.Adam
+ * (step 1: z - lr*g/(|g|+1e-8)) or SGD (z - lr*g).  Iteration 1 reads z_mean, later ones the
+ * previous iteration's z; the Adam moments of a multi-step call live in the handle ([max_rows,T,4]
+ * x 2, allocated by the first call with grad_steps > 1).  cond/curr are per ROW ([R,C], [R,4]).
+ * grad_out [R,T,4] and loss_out [7,R] (agent_collision, map_collision, target_pos, target_speed,
+ * acc_limit, speed_limit, waypoint per row) may be NULL; with grad_steps > 1 they hold the gradient
+ * and the losses of the LAST iteration, as perturb returns them.  z_out may alias z_mean. */
 int cld_guidance_step(CldHandle* h, const float* z_mean, const float* cond, const float* curr,
                       const CldScene* scene, const CldGuidanceConfig* g, float* z_out,
                       float* grad_out, float* loss_out, int R, void* stream);
@@ -242,7 +247,8 @@ int cld_guidance_step(CldHandle* h, const float* z_mean, const float* cond, cons
  *   Philox4x32-10 noise.  row_offset = GLOBAL id of row 0 of this call (0 for an unsharded call): the Philox
  *   counter of an element is (global row, element, step), so a shard / chunk / lane of a batch draws exactly
  *   what the unsharded batch would (SURVEY.md sec. 8e).
- *   cond [R,C], curr [R,4] per row; scene/g may be NULL (unguided, no indicators).
+ *   cond [R,C], curr [R,4] per row; scene/g may be NULL (unguided, no indicators).  Every guided
+ *   step runs the g->grad_steps iterations of cld_guidance_step on the posterior mean.
  * Outputs (any may be NULL): x0 [R,T,D], x1 [R,T,D] (written only if step index 1 is visited;
  * *x1_valid says so), traj [R,T,6], offroad [R,T], coll [R]. */
 int cld_sample(CldHandle* h, const float* x_init, const float* noises, uint64_t seed,
