@@ -247,10 +247,11 @@ int cld_create(const CldConfig* cfg, CldHandle** out) {
   if (cfg->max_rows < 1) return fail(nullptr, CLD_ERR_ARG, "max_rows must be positive");
   if (cfg->n_timesteps < 1) return fail(nullptr, CLD_ERR_ARG, "n_timesteps must be positive");
   {
-    const bool t_ok = (cfg->horizon >= 16 && cfg->horizon <= 56) || (cfg->horizon >= 64 && cfg->horizon <= 112 && cfg->horizon % 8 == 0);
+    TcLevel levels[3];
+    const bool t_ok = tc_level_layout(cfg->horizon, levels);      // the horizons tc_finalize can lay out, no others
     if (cfg->precision == CLD_PREC_BF16 && !(cfg->dims[0] == 64 && cfg->dims[1] == 128 && cfg->dims[2] == 256 && t_ok && cfg->hidden == 64))
       return fail(nullptr, CLD_ERR_UNSUPPORTED,
-                  "the bf16 tensor-core path is built for dims (64,128,256), hidden 64 and a horizon of 16..56 (8 rows per CTA) or 64..112 in "
+                  "the bf16 tensor-core path is built for dims (64,128,256), hidden 64 and a horizon of 16..56 (8 rows per CTA) or 64..104 in "
                   "multiples of 8 (4 rows per CTA as two half-horizon lanes); use precision fp32 for this configuration");
   }
   CldHandle* h = new CldHandle();

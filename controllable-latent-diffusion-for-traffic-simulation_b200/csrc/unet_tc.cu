@@ -858,8 +858,37 @@ __global__ void tc_copy_scale_kernel(float* __restrict__ dst, const float* __res
 
 static TcState* st_of(CldHandle* h) { return reinterpret_cast<TcState*>(h->tc); }
 
+bool tc_level_layout(int horizon, TcLevel L[3]) {
+  // 8-row mode covers 16..56 steps; above that each row runs as two lanes of horizon / 2 steps, which must be a multiple of 4 so
+  // that every level of a lane has a whole number of slots
+  const bool tsplit = horizon > 56;
+  if (horizon < 16 || horizon % 4 || (tsplit && horizon % 8)) return false;
+  const int T = tsplit ? horizon / 2 : horizon;
+  const int np[3] = {1, 2, 4};
+  for (int l = 0; l < 3; ++l) {
+    TcLevel& v = L[l];
+    v.T = T >> l; v.npanels = np[l];
+    // 8-row mode: the 2 halo slots between two panels are shared (both zero); split-time mode: every panel has its own leading and
+    // trailing halo, because the inner one carries the partner lane's edge slots
+    if (tsplit) { v.pitch = (v.T + 4) * 1024; v.offB = np[l] * v.pitch; }
+    else { v.pitch = (v.T + 2) * 1024; v.offB = np[l] * v.pitch + 2048; }
+    v.n_tiles = (v.T + 15) / 16;
+    for (int i = 0; i < 4; ++i) { v.slot0[i] = 0; v.lo[i] = 0; v.hi[i] = 0; }
+    for (int i = 0; i < v.n_tiles; ++i) {
+      bool last = i == v.n_tiles - 1;
+      v.slot0[i] = (last && v.T >= 16) ? v.T - 16 : 16 * i;
+      v.lo[i] = 16 * i - v.slot0[i];
+      v.hi[i] = (v.T - v.slot0[i] < 16) ? v.T - v.slot0[i] : 16;
+    }
+    // every 16-slot tile read (plus taps, plus stride-2 reads from the level above) must stay inside the arena
+    // (split-time mode: the regions fill the arena exactly; the reads of masked rows past its end land in the weight ring)
+    if (tsplit ? (v.offB + v.npanels * v.pitch > TC_ARENA) : (v.offB + v.npanels * v.pitch + 5 * 1024 > TC_ARENA)) return false;
+  }
+  return true;
+}
+
 namespace {
-struct Level { int T, pitch, offB, npanels, n_tiles, slot0[4], lo[4], hi[4]; };
+using Level = TcLevel;
 
 struct ConvSpec {          // one convolution (or one output phase of a transposed convolution)
   const float* w; int cout, cin, K, transposed;
@@ -928,28 +957,8 @@ int tc_finalize(CldHandle* h, const float* const* p, cudaStream_t stream) {
   const int T = s->tsplit ? c.horizon / 2 : c.horizon;
   s->t_eff = T;
   Level L[3];
-  const int np[3] = {1, 2, 4};
-  for (int l = 0; l < 3; ++l) {
-    Level& v = L[l];
-    v.T = T >> l; v.npanels = np[l];
-    // 8-row mode: the 2 halo slots between two panels are shared (both zero); split-time mode: every panel has its own leading and
-    // trailing halo, because the inner one carries the partner lane's edge slots
-    if (s->tsplit) { v.pitch = (v.T + 4) * 1024; v.offB = np[l] * v.pitch; }
-    else { v.pitch = (v.T + 2) * 1024; v.offB = np[l] * v.pitch + 2048; }
-    v.n_tiles = (v.T + 15) / 16;
-    for (int i = 0; i < 4; ++i) { v.slot0[i] = 0; v.lo[i] = 0; v.hi[i] = 0; }
-    for (int i = 0; i < v.n_tiles; ++i) {
-      bool last = i == v.n_tiles - 1;
-      v.slot0[i] = (last && v.T >= 16) ? v.T - 16 : 16 * i;
-      v.lo[i] = 16 * i - v.slot0[i];
-      v.hi[i] = (v.T - v.slot0[i] < 16) ? v.T - v.slot0[i] : 16;
-    }
-    // every 16-slot tile read (plus taps, plus stride-2 reads from the level above) must stay inside the arena
-    // (split-time mode: the regions fill the arena exactly; the reads of masked rows past its end land in the weight ring)
-    if (s->tsplit ? (v.offB + v.npanels * v.pitch > TC_ARENA) : (v.offB + v.npanels * v.pitch + 5 * 1024 > TC_ARENA))
-      return fail(h, CLD_ERR_UNSUPPORTED, "horizon too long for the bf16 arena");
-    if (l == 0) { s->zero0_pitch = v.pitch; s->zero0_offB = v.offB; }
-  }
+  if (!tc_level_layout(c.horizon, L)) return fail(h, CLD_ERR_UNSUPPORTED, "horizon too long for the bf16 arena");
+  s->zero0_pitch = L[0].pitch; s->zero0_offB = L[0].offB;
   Builder B{s};
   s->ops.clear(); s->kbs.clear();
   const int k5[5] = {0, 1, 2, 3, 4}, o5[5] = {-2, -1, 0, 1, 2}, k1[1] = {0}, o1[1] = {0};
