@@ -86,63 +86,105 @@ __device__ __forceinline__ float target_pos_term(const float* __restrict__ tr, f
   return E / (float)Tn;
 }
 
+__device__ __forceinline__ bool is_moving(const LossArgs& a, size_t g) { return fabsf(a.speed[g]) > a.speed_th; }
+
+// Agent-collision constants of agent g (its global agent index): rad, cmin, cmax, moving, R00, R01, R10, R11
+__device__ __forceinline__ void collision_consts(const LossArgs& a, size_t g, float* q) {
+  float L = a.extent[g * 3 + 0], Wd = a.extent[g * 3 + 1];
+  float rad = Wd / 2.f;
+  q[0] = rad; q[1] = -(L / 2.f) + rad; q[2] = (L / 2.f) - rad;
+  q[3] = is_moving(a, g) ? 1.f : 0.f;
+  q[4] = a.wfa[g * 9 + 0]; q[5] = a.wfa[g * 9 + 1]; q[6] = a.wfa[g * 9 + 3]; q[7] = a.wfa[g * 9 + 4];
+}
+
+// World pose (Px, Py, cos Psi, sin Psi) of agent g, sample n at step t: transform_agents_to_world (geometry_utils.py:458-483)
+__device__ __forceinline__ float4 world_pose(const LossArgs& a, size_t g, int n, int t) {
+  const float* tr = a.traj + ((g * a.N + n) * a.T + t) * 6;
+  float px = tr[0], py = tr[1], psi = tr[3];
+  const float* M = a.wfa + g * 9;
+  float Px = M[0] * px + M[1] * py + M[2], Py = M[3] * px + M[4] * py + M[5];
+  float c = cosf(psi), sn = sinf(psi);
+  float hx = M[0] * c + M[1] * sn, hy = M[3] * c + M[4] * sn;
+  float Psi = atan2f(hy, hx);
+  return make_float4(Px, Py, cosf(Psi), sinf(Psi));
+}
+
+// Stage partners [g0, g0 + nt) of sample n at steps [t0, t0 + nts): poses [nt][ts][4] (ts >= nts steps per partner) and
+// constants [nt][8]
+__device__ __forceinline__ void stage_partners(const LossArgs& a, float* pose, float* agt, size_t g0, int nt, int n, int t0, int nts,
+                                               int ts) {
+  const int tid = threadIdx.x, nthr = blockDim.x;
+  for (int j = tid; j < nt; j += nthr) collision_consts(a, g0 + j, agt + j * 8);
+  for (int it = tid; it < nt * nts; it += nthr) {
+    const int j = it / nts, t = it - j * nts;
+    reinterpret_cast<float4*>(pose)[(size_t)j * ts + t] = world_pose(a, g0 + j, n, t0 + t);
+  }
+}
+
+// Agent-collision partners in shared memory: a scene of up to SCENE_TILE agents is staged whole, a larger one streams tiles of
+// PARTNER_TILE agents x 32 steps
+constexpr int SCENE_TILE = 64, PARTNER_TILE = 128;
+
 __global__ void __launch_bounds__(512) guidance_loss_grad_kernel(LossArgs a) {
   extern __shared__ __align__(16) float sm[];
   const int A = a.A, T = a.T, N = a.N;
-  float* pose = sm;                         // [A][T][4] world Px, Py, cos(Psi), sin(Psi)
-  float* agt = pose + (size_t)A * T * 4;    // [A][8]: rad, cmin, cmax, moving, R00, R01, R10, R11
-  float* wts = agt + A * 8;                 // [T] decay weights
+  // The partners j of the agent-collision term pass through shared memory in tiles.  A scene of at most SCENE_TILE agents is
+  // one tile holding all its steps, staged once.  A larger scene is streamed as tiles of PARTNER_TILE partners x the 32 steps
+  // of one lane slot, so shared memory does not depend on A.  Tiles go in ascending j: every sum over partners is added in the
+  // same order whatever the tiling.
+  const bool one_tile = A <= SCENE_TILE;
+  const int P = one_tile ? A : PARTNER_TILE, TS = one_tile ? T : 32;
+  float* pose = sm;                         // [P][TS][4] world Px, Py, cos(Psi), sin(Psi) of the tile's partners
+  float* agt = pose + (size_t)P * TS * 4;   // [P][8]: rad, cmin, cmax, moving, R00, R01, R10, R11
+  float* wts = agt + P * 8;                 // [T] decay weights
   const int s = blockIdx.x / N, n = blockIdx.x % N;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int nthr = blockDim.x, nwarps = nthr >> 5;       // 16 warps: one agent per warp at 16 agents per scene (latency-bound loops: more warps per SM)
   // the agents of a scene are dealt to gridDim.y CTAs (large scenes: 64 agents x 104 steps x 63 partners would otherwise sit on
-  // S * N CTAs); every CTA stages the poses of ALL agents (the partners) and evaluates the terms of agents [i_lo, i_hi)
+  // S * N CTAs); every CTA visits the poses of ALL agents (the partners) and evaluates the terms of agents [i_lo, i_hi)
   const int per_cta = (A + (int)gridDim.y - 1) / (int)gridDim.y;
   const int i_lo = (int)blockIdx.y * per_cta, i_hi = min(A, i_lo + per_cta);
-  const int ag0 = s * A;
+  const size_t ag0 = (size_t)s * A;
   const float inv_AN = 1.0f / (float)(A * N);
 
-  if (tid < A) {
-    const int g = ag0 + tid;
-    float L = a.extent[g * 3 + 0], Wd = a.extent[g * 3 + 1];
-    float rad = Wd / 2.f;
-    float* q = agt + tid * 8;
-    q[0] = rad; q[1] = -(L / 2.f) + rad; q[2] = (L / 2.f) - rad;
-    q[3] = (fabsf(a.speed[g]) > a.speed_th) ? 1.f : 0.f;
-    q[4] = a.wfa[g * 9 + 0]; q[5] = a.wfa[g * 9 + 1]; q[6] = a.wfa[g * 9 + 3]; q[7] = a.wfa[g * 9 + 4];
-  }
   for (int t = tid; t < T; t += nthr) wts[t] = a.wts[t];
-  for (int it = tid; it < A * T; it += nthr) {
-    int i = it / T, t = it - i * T, g = ag0 + i;
-    const float* tr = a.traj + (((size_t)g * N + n) * T + t) * 6;
-    float px = tr[0], py = tr[1], psi = tr[3];
-    const float* M = a.wfa + (size_t)g * 9;
-    // transform_agents_to_world (geometry_utils.py:458-483)
-    float Px = M[0] * px + M[1] * py + M[2], Py = M[3] * px + M[4] * py + M[5];
-    float c = cosf(psi), sn = sinf(psi);
-    float hx = M[0] * c + M[1] * sn, hy = M[3] * c + M[4] * sn;
-    float Psi = atan2f(hy, hx);
-    float* p = pose + (size_t)it * 4;
-    p[0] = Px; p[1] = Py; p[2] = cosf(Psi); p[3] = sinf(Psi);
-  }
+  if (one_tile) stage_partners(a, pose, agt, ag0, A, n, 0, T, T);
   __syncthreads();
 
   // ---------------- agent-agent collision: warp per agent, lanes over time ---------------------
-  for (int i = i_lo + warp; i < i_hi; i += nwarps) {
-    const int g = ag0 + i;
-    const size_t row = (size_t)g * N + n;
-    const float* qi = agt + i * 8;
+  // Loops that stage tiles are CTA-uniform: every warp runs all rounds and slots.  With several tiles the host deals at most one
+  // agent to a warp (one round), so each tile is staged once per CTA.
+  const int rounds = i_hi > i_lo ? (i_hi - i_lo + nwarps - 1) / nwarps : 0;
+  for (int r = 0; r < rounds; ++r) {
+    const int i = i_lo + r * nwarps + warp;
+    const bool active = i < i_hi;                        // warp-uniform
+    const size_t g = ag0 + (active ? i : i_lo);
+    const size_t row = g * N + n;
+    float qi[8];
+    collision_consts(a, g, qi);
     const float rad_i = qi[0], mov_i = qi[3];
     float loss_i = 0.f;
-    for (int t = lane; t < T; t += 32) {
+    for (int t0 = 0; t0 < T; t0 += 32) {
+      const int t = t0 + lane;
+      const bool live = active && t < T;
       float gPx = 0.f, gPy = 0.f, gPsi = 0.f, pen_sum = 0.f;
-      if (a.w_ac != 0.f) {
-        const float* pi = pose + ((size_t)i * T + t) * 4;
-        const float Pix = pi[0], Piy = pi[1], ci = pi[2], si = pi[3];
-        for (int j = 0; j < A; ++j) {
-          if (j == i) continue;
-          const float* qj = agt + j * 8;
-          const float* pj = pose + ((size_t)j * T + t) * 4;
+      // agent i's own pose: from the staged scene, or evaluated here
+      float4 pi = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (live && a.w_ac != 0.f) pi = one_tile ? reinterpret_cast<const float4*>(pose)[(size_t)i * T + t] : world_pose(a, g, n, t);
+      const float Pix = pi.x, Piy = pi.y, ci = pi.z, si = pi.w;
+      for (int j0 = 0; j0 < A; j0 += P) {
+        const int nt = min(P, A - j0);
+        if (!one_tile) {
+          __syncthreads();                               // the previous tile is no longer read
+          stage_partners(a, pose, agt, ag0 + j0, nt, n, t0, min(32, T - t0), TS);
+          __syncthreads();
+        }
+        if (!live || a.w_ac == 0.f) continue;
+        const int tt = one_tile ? t : lane;
+        for (int jj = 0; jj < nt; ++jj) {
+          if (j0 + jj == i) continue;
+          const float* qj = agt + jj * 8;
+          const float* pj = pose + ((size_t)jj * TS + tt) * 4;
           float pd = rad_i + qj[0] + a.buffer;
           {
             // the disk centres lie within reach_i / reach_j of the agents' centres: when the centres are further apart than
@@ -174,22 +216,24 @@ __global__ void __launch_bounds__(512) guidance_loss_grad_kernel(LossArgs a) {
           }
         }
       }
+      if (!live) continue;
       const float wt = wts[t];
       float kk = a.w_ac * inv_AN * (1.0f / (float)A) * wt;
       gPx *= kk; gPy *= kk; gPsi *= kk;
       // back to the agent frame: p = R^T P ; dPsi/dpsi through atan2(R [cos, sin])
-      const float* tr = a.traj + ((size_t)row * T + t) * 6;
+      const float* tr = a.traj + (row * T + t) * 6;
       float psi = tr[3], c = cosf(psi), sn = sinf(psi);
       float hx = qi[4] * c + qi[5] * sn, hy = qi[6] * c + qi[7] * sn;
       float dhx = -qi[4] * sn + qi[5] * c, dhy = -qi[6] * sn + qi[7] * c;
       float dPsi_dpsi = (hx * dhy - hy * dhx) / (hx * hx + hy * hy);
-      float* o = a.dtraj + ((size_t)row * T + t) * 4;
+      float* o = a.dtraj + (row * T + t) * 4;
       o[0] = qi[4] * gPx + qi[6] * gPy;
       o[1] = qi[5] * gPx + qi[7] * gPy;
       o[2] = 0.f;
       o[3] = gPsi * dPsi_dpsi;
       loss_i += wt * pen_sum;
     }
+    if (!active) continue;
 #pragma unroll
     for (int o = 16; o; o >>= 1) loss_i += __shfl_xor_sync(0xffffffffu, loss_i, o);
     if (lane == 0 && a.loss) a.loss[row] = (mov_i != 0.f) ? loss_i / (float)A : 0.f;
@@ -203,10 +247,10 @@ __global__ void __launch_bounds__(512) guidance_loss_grad_kernel(LossArgs a) {
   if (a.w_tp != 0.f && a.target) {
     const int t0 = (int)(a.min_target_time * (float)T);
     for (int i = i_lo + warp; i < i_hi; i += nwarps) {
-      const int g = ag0 + i;
+      const size_t g = ag0 + i;
       const size_t row = (size_t)g * N + n;
       // stationary agents were detached in place by the agent-collision term (guidance_loss.py:511-515)
-      const bool has_grad = !(a.w_ac != 0.f && agt[i * 8 + 3] == 0.f);
+      const bool has_grad = !(a.w_ac != 0.f && !is_moving(a, g));
       const float l = target_pos_term(a.traj + (size_t)row * T * 6, a.dtraj + (size_t)row * T * 4, a.target[g * 2 + 0], a.target[g * 2 + 1], t0, T,
                                       lane, has_grad ? a.w_tp * inv_AN : 0.f);
       if (lane == 0 && a.loss) a.loss[2 * (size_t)a.R + row] = l;
@@ -221,10 +265,10 @@ __global__ void __launch_bounds__(512) guidance_loss_grad_kernel(LossArgs a) {
   //   GlobalTargetPosLoss (:1033-1135) with compute_progress_loss (:876-927); which branch an agent takes is host logic (wp_mode)
   if (a.w_wp != 0.f && a.wp_mode) {
     for (int i = i_lo + warp; i < i_hi; i += nwarps) {
-      const int g = ag0 + i;
+      const size_t g = ag0 + i;
       const size_t row = (size_t)g * N + n;
       const int mode = a.wp_mode[g];
-      const bool has_grad = !(a.w_ac != 0.f && agt[i * 8 + 3] == 0.f);
+      const bool has_grad = !(a.w_ac != 0.f && !is_moving(a, g));
       const float kk = has_grad ? a.w_wp * inv_AN * (a.wp_w ? a.wp_w[g] : 1.f) : 0.f;
       const float* tr = a.traj + (size_t)row * T * 6;
       float* dt_ = a.dtraj + (size_t)row * T * 4;
@@ -270,9 +314,9 @@ __global__ void __launch_bounds__(512) guidance_loss_grad_kernel(LossArgs a) {
   if (any_sp || a.loss) {
     const float invT = 1.0f / (float)T;
     for (int i = i_lo + warp; i < i_hi; i += nwarps) {
-      const int g = ag0 + i;
+      const size_t g = ag0 + i;
       const size_t row = (size_t)g * N + n;
-      const bool has_grad = !(a.w_ac != 0.f && agt[i * 8 + 3] == 0.f);     // in-place detach of stationary agents, as above
+      const bool has_grad = !(a.w_ac != 0.f && !is_moving(a, g));     // in-place detach of stationary agents, as above
       const float* tr = a.traj + (size_t)row * T * 6;
       float l_ts = 0.f, l_al = 0.f, l_sl = 0.f;
       for (int t = lane; t < T; t += 32) {
@@ -622,7 +666,7 @@ int guidance_loss_grad(CldHandle* h, const float* traj, const CldScene* sc, cons
   int rc;
   const int S = sc->num_scenes, A = sc->agents_per_scene, N = sc->num_samp, T = h->cfg.horizon;
   if (R != S * A * N) return fail(h, CLD_ERR_ARG, "R=%d does not match S*A*N=%d*%d*%d", R, S, A, N);
-  if (A < 1 || A > 64) return fail(h, CLD_ERR_UNSUPPORTED, "agents_per_scene must be in [1,64]");
+  if (A < 1) return fail(h, CLD_ERR_UNSUPPORTED, "agents_per_scene must be >= 1");
   if (g->num_disks < 1 || g->num_disks > 5) return fail(h, CLD_ERR_UNSUPPORTED, "num_disks must be in [1,5]");
   if (g->num_points_l < 1 || g->num_points_l > 16 || g->num_points_w < 1 || g->num_points_w > 16 ||
       g->num_points_l * g->num_points_w > 128)
@@ -661,7 +705,9 @@ int guidance_loss_grad(CldHandle* h, const float* traj, const CldScene* sc, cons
     for (int t = 0; t < T; ++t) a.wts[t] /= sum;
     for (int t = T; t < CLD_MAX_T; ++t) a.wts[t] = 0.f;
   }
-  size_t smem = ((size_t)A * T * 4 + (size_t)A * 8 + T) * sizeof(float);
+  // the whole scene (at most 133 KB: A = 64, T = 128), or one tile of partners (65 KB and the decay weights)
+  const bool one_tile = A <= SCENE_TILE;
+  const size_t smem = ((size_t)(one_tile ? A : PARTNER_TILE) * ((one_tile ? T : 32) * 4 + 8) + T) * sizeof(float);
   CLD_CUDA_OK(h, cudaFuncSetAttribute(guidance_loss_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const bool fork = dtraj_map != nullptr && loss == nullptr && a.w_mc != 0.f;
   if (fork) {
@@ -681,7 +727,15 @@ int guidance_loss_grad(CldHandle* h, const float* traj, const CldScene* sc, cons
   }
   // enough CTAs for ~2 per SM: the agents of a scene are split over gridDim.y CTAs when there are few (scene, sample) pairs
   int split = 1;
-  while (S * N * split < 2 * h->num_sms && split * 2 <= (A + 3) / 4) split *= 2;
+  if (one_tile) {
+    while (S * N * split < 2 * h->num_sms && split * 2 <= (A + 3) / 4) split *= 2;
+  } else {
+    // several tiles: at most one agent per warp (16 per CTA), so a CTA stages each tile once; down to 4 agents per CTA while
+    // the grid is short of 2 CTAs per SM
+    int per = 16;
+    while (per > 4 && (size_t)S * N * ((A + per - 1) / per) < 2 * (size_t)h->num_sms) per /= 2;
+    split = (A + per - 1) / per;
+  }
   const int per_cta = (A + split - 1) / split;
   const int threads = 32 * (per_cta < 4 ? 4 : (per_cta > 16 ? 16 : per_cta));       // one warp per agent, 4 .. 16 warps
   guidance_loss_grad_kernel<<<dim3((unsigned)(S * N), (unsigned)split), threads, smem, s>>>(a);

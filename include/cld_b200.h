@@ -91,7 +91,7 @@ typedef struct {
 /* Per-agent scene tensors (the reference's data_batch entries), B = S*A agent rows, scene-major. */
 typedef struct {
   int32_t num_scenes;               /* S */
-  int32_t agents_per_scene;         /* A (<= 64) */
+  int32_t agents_per_scene;         /* A >= 1; any size is guided: one scene's A*N rows must fit CldConfig.max_rows */
   int32_t num_samp;                 /* N */
   const float* extent;              /* [B,3]  data_batch['extent']                               */
   const float* world_from_agent;    /* [B,3,3]                                                   */
