@@ -702,12 +702,16 @@ static int train_prepare(CldHandle* h, int R) {
   }
   if (tb_total > CLD_TB_TOTAL_MAX) return fail(h, CLD_ERR_UNSUPPORTED, "time-bias width %d above %d", tb_total, CLD_TB_TOTAL_MAX);
   if (td > 64) return fail(h, CLD_ERR_UNSUPPORTED, "the denoiser backward needs base_dim <= 64");
+  // every buffer starts on a 16-byte boundary whatever the row count (float4 loads and TMA need it): per-row sizes are rounded up to
+  // a multiple of 4 floats
+  auto r4 = [](size_t n) { return (n + 3) & ~(size_t)3; };
   // 12 blocks x 4 + p0 p1 q0 q1 fA fB tmpR + gB + 2 x 2 (concat gradients) = 60 E, + 26 dA + 20 data-gradient buffers, + the small per-row vectors
-  const size_t per_row = (60 + TrainState::MAX_UNITS + TrainState::MAX_GD) * E + (size_t)TrainState::MAX_UNITS * 768 + (size_t)tb_total + 64 + td + 4 * td + 4 * td + td + 1 + (size_t)c.horizon * c.latent_dim;
+  const size_t per_row = (60 + TrainState::MAX_UNITS + TrainState::MAX_GD) * r4(E) + (size_t)TrainState::MAX_UNITS * 768 + r4(tb_total) + 64 +
+                         r4(td) + 4 * r4(td) + 4 * r4(td) + r4(td) + r4(1) + r4((size_t)c.horizon * c.latent_dim);
   const size_t cap = (size_t)R;
   CLD_CUDA_OK(h, cudaMalloc((void**)&st->arena, per_row * cap * sizeof(float)));
   float* p = st->arena;
-  auto take = [&](size_t per) { float* q = p; p += per * cap; return q; };
+  auto take = [&](size_t per) { float* q = p; p += r4(per) * cap; return q; };
   for (int b = 0; b < 12; ++b) { st->blk[b].A0 = take(E); st->blk[b].B0 = take(E); st->blk[b].A1 = take(E); st->blk[b].OUT = take(E); }
   st->p0 = take(E); st->p1 = take(E); st->q0 = take(E); st->q1 = take(E); st->fA = take(E); st->fB = take(E); st->tmpR = take(E);
   st->gB = take(E); st->gcat8 = take(2 * E); st->gcat10 = take(2 * E);

@@ -111,7 +111,9 @@ def unet_forward(sd, x, cond, t, taps=None):
     activations after every stage, channels-last [R,T',C], for per-layer kernel debugging.
     """
     h = x.transpose(1, 2)
-    te = sinusoid(t, sd['time_mlp.1.weight'].shape[1])
+    # the embedding is computed in float32 (as the reference and the kernels do), then follows the weights' dtype: a float64 state
+    # dict gives a float64 forward, a float32 one is unchanged
+    te = sinusoid(t, sd['time_mlp.1.weight'].shape[1]).to(sd['time_mlp.1.weight'].dtype)
     te = F.linear(te, sd['time_mlp.1.weight'], sd['time_mlp.1.bias'])
     te = F.linear(mish(te), sd['time_mlp.3.weight'], sd['time_mlp.3.bias'])
     tc = torch.cat([te, cond], dim=-1)

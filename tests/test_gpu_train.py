@@ -260,36 +260,32 @@ def test_compute_losses_mse_vs_reference_golden(dm16, gold):
 
 def test_graph_replay_equals_eager_updates(models_cpu, gold):
     """GraphedPPOStep (the update captured as a CUDA graph: two streams inside, device-side baseline / lr / step) reproduces the
-    parameters of the same sequence of un-captured updates bit for bit."""
-    from cld_b200.trainer import FusedAdam, GraphedPPOStep
-    g = gold("ppo")
-    finals = []
-    for use_graph in (False, True):
-        dm, _, _ = models_cpu(16)
-        dm = dm.cuda()
-        dm.train_precision = "tf32"
-        for p in dm.model.parameters():
-            p.requires_grad_(True)
-        opt = FusedAdam(dm, lr=1e-4, weight_decay=1e-5)
-        x1, x0, cond, t, lp_old, reward, baseline, clip = _ppo_inputs(g)
-        gs = GraphedPPOStep(dm, opt, x1.shape[0], clip) if use_graph else None
-        losses = []
-        for it in range(6):
-            xs = x1 + 0.01 * it                                   # a different minibatch every iteration
-            base = baseline + 0.1 * (it // 3)                     # the baseline and the learning rate change between replays
-            opt.lr = 1e-4 * (1.0 if it < 4 else 0.5)
-            if use_graph:
-                for dst, src in zip(gs.buffers(), (x0, xs, lp_old, reward, cond)):
-                    dst.copy_(src)
-                losses.append(float(gs(base, t)))
-            else:
-                loss, _ = dm.ppo_minibatch_grad(xs, x0, cond, t, lp_old, reward, base, clip)
-                opt.step()
-                losses.append(float(loss))
-        assert opt.step_count == 6
-        finals.append((losses, dm._flat.clone()))
-    assert finals[0][0] == finals[1][0], (finals[0][0], finals[1][0])
-    assert torch.equal(finals[0][1], finals[1][1])
+    parameters of the same sequence of un-captured updates bit for bit (tests/ppo_cases.py; six updates of the golden minibatch)."""
+    from ppo_cases import assert_graph_replay_equals_eager
+    x1, x0, cond, t, lp_old, reward, baseline, clip = _ppo_inputs(gold("ppo"))
+    assert_graph_replay_equals_eager(lambda: models_cpu(16)[0].cuda(), x1, x0, cond, t, lp_old, reward, baseline, clip, iters=6)
+
+
+def test_ppo_minibatch_odd_rows_vs_float64_oracle(dm16):
+    """cld_ppo_grad on a training arena carved for 37 rows: a row count that is not a multiple of 4 must leave every arena buffer
+    16-byte aligned (the head's d_eps feeds float4 loads of the output convolution's backward).  log_p_new, loss and all 148 gradients
+    against O.ppo_grads in float64 (fp32 mode)."""
+    from ppo_cases import clip_regions, ppo_case, ppo_oracle
+    dm, _, _ = dm16
+    R, baseline, clip = 37, 0.05, 0.2
+    sd64 = {k: v.detach().cpu().double() for k, v in dm.model.state_dict().items()}
+    sched = {k: v.detach().cpu().double() for k, v in dm.named_buffers()}
+    case = ppo_case(sched, sd64, R, 37)
+    loss_want, lp_want, g_want = ppo_oracle(sd64, sched, *case, baseline, clip)
+    inside, cut = clip_regions(lp_want, case[4], case[5], baseline, clip)
+    assert inside.any() and cut.any()
+    loss, lp = dm.ppo_minibatch_grad(*(v.cuda() for v in case[:4]), case[4].cuda(), case[5].cuda(), baseline, clip)
+    assert rel(lp, lp_want) < 1e-5
+    assert abs(float(loss) - loss_want) < 1e-5 * max(1.0, abs(loss_want))
+    errs = {k: rel(g, w) for k, g, w in zip(dm.model.state_dict(), dm._flat_views[1], g_want)}
+    bad = {k: v for k, v in errs.items() if not v < GRAD_TOL}
+    assert not bad, bad
+    print("R=37 fp32 PPO minibatch: log_p_new rel %.2e, worst gradient %.2e" % (rel(lp, lp_want), max(errs.values())))
 
 
 def test_adam_kernel_vs_torch(dm16):

@@ -255,6 +255,32 @@ def test_ppo_oracle_vs_reference_golden(gold, models_cpu):
     assert (got[big] - torch.tensor(g["delta_samples"][7]).double()[big]).abs().max().item() < 2e-2 * float(g["lr"])
 
 
+def test_oracle_runs_in_float64(models_cpu):
+    """The float64 oracle is the reference of the large-batch training tests (tests/test_gpu_train_large.py): the U-Net forward
+    and the PPO gradients take a float64 state dict, agree with the float32 oracle, and return float64 everywhere."""
+    dm, _, _ = models_cpu(16)
+    sd32 = {k: v.detach() for k, v in dm.model.state_dict().items()}
+    sd64 = {k: v.double() for k, v in sd32.items()}
+    torch.manual_seed(11)
+    R = 5
+    x, cond, t = torch.randn(R, 52, 4), torch.randn(R, 256), torch.randint(0, 16, (R,))
+    with torch.no_grad():
+        e32 = O.unet_forward(sd32, x, cond, t)
+        e64 = O.unet_forward(sd64, x.double(), cond.double(), t)
+    assert e32.dtype == torch.float32 and e64.dtype == torch.float64
+    assert rel(e32, e64) < 1e-6
+    sched64 = {k: v.double() for k, v in O.make_schedule(16).items()}
+    t = torch.randint(1, 16, (R,))
+    x0 = torch.randn(R, 52, 4, dtype=torch.float64)
+    lp_old, reward = -torch.rand(R, dtype=torch.float64), torch.randn(R, dtype=torch.float64)
+    loss, lp, grads = O.ppo_grads(sd64, sched64, x.double(), x0, cond.double(), t, lp_old, reward, 0.1, 0.2)
+    assert loss.dtype == lp.dtype == torch.float64 and all(g.dtype == torch.float64 for g in grads.values())
+    assert list(grads) == list(sd64) and torch.isfinite(lp).all()
+    loss32, lp32, grads32 = O.ppo_grads(sd32, O.make_schedule(16), x, x0.float(), cond, t, lp_old.float(), reward.float(), 0.1, 0.2)
+    assert rel(lp32, lp) < 1e-5
+    assert max(rel(grads32[k], grads[k]) for k in grads) < 1e-3
+
+
 def test_warmup_cosine_schedule():
     """lr factor of configure_optimizers (guide_dm_trainer.py:67-75)."""
     from cld_b200.trainer import warmup_cosine
