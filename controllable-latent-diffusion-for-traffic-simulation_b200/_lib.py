@@ -54,6 +54,7 @@ class CldScene(C.Structure):
         ("target_pos", C.c_void_p), ("others_pos", C.c_void_p), ("others_avail", C.c_void_p),
         ("num_others", C.c_int32), ("map_packed", C.c_int32), ("target_speed", C.c_void_p),
         ("wp_target", C.c_void_p), ("wp_mode", C.c_void_p), ("wp_time", C.c_void_p), ("wp_dist", C.c_void_p), ("wp_weight", C.c_void_p),
+        ("scene_start", C.c_void_p), ("scene_start_host", C.c_void_p),
     ]
 
 

@@ -4,32 +4,17 @@ import torch
 
 @torch.no_grad()
 def indicators(dm, state_action, batch, num_samp=1):
-    """Per-row indicators: offroad [R,T] bool, collision counts [R], reward [R].  Ragged batches (scenes of different sizes) are
-    evaluated as one uniform sub-batch per scene size (`keys.scene_buckets`)."""
-    from .keys import scene_buckets, scene_sizes
+    """Per-row indicators: offroad [R,T] bool, collision counts [R], reward [R].  Scenes may differ in size (`scene_index`): the
+    batch is evaluated in one call either way."""
+    from .keys import scene_sizes
     R = state_action.shape[0]
     x = state_action
     if x.shape[-1] < 6:
         x = torch.cat([x, x.new_zeros(*x.shape[:-1], 6 - x.shape[-1])], dim=-1)
     B = R // num_samp
     sizes = scene_sizes(batch.get('scene_index'), B)
-    if len(set(sizes)) == 1:
-        A = sizes[0]
-        return dm.engine(R).indicators(x, dm.engine(R).make_scene(batch, B // A, A, num_samp))
-    outs = None
-    for A, idx in scene_buckets(sizes):
-        idx = idx.to(x.device)
-        rows = (idx[:, None] * num_samp + torch.arange(num_samp, device=x.device)[None, :]).reshape(-1)
-        nb = idx.numel()
-        sub = {k: (v.index_select(0, idx.to(v.device)) if (torch.is_tensor(v) and v.dim() > 0 and v.shape[0] == B) else v) for k, v in batch.items()}
-        sub['scene_index'] = torch.arange(nb // A).repeat_interleave(A)
-        eng = dm.engine(nb * num_samp)
-        o = eng.indicators(x.index_select(0, rows), eng.make_scene(sub, nb // A, A, num_samp))
-        if outs is None:
-            outs = [v.new_empty((R,) + tuple(v.shape[1:])) for v in o]
-        for dst, v in zip(outs, o):
-            dst.index_copy_(0, rows, v)
-    return tuple(outs)
+    eng = dm.engine(R)
+    return eng.indicators(x, eng.make_scene(batch, len(sizes), sizes[0], num_samp, scene_sizes=sizes))
 
 
 @torch.no_grad()

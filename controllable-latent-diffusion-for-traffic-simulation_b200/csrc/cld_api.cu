@@ -214,6 +214,27 @@ static int unet_setup(CldHandle* h) {
   return 0;
 }
 
+int check_scene(CldHandle* h, const CldScene* sc, int R) {
+  const int S = sc->num_scenes, N = sc->num_samp;
+  if (S < 1 || N < 1) return fail(h, CLD_ERR_ARG, "num_scenes=%d and num_samp=%d must be >= 1", S, N);
+  if (!sc->scene_start && !sc->scene_start_host) {
+    const int A = sc->agents_per_scene;
+    if (A < 1) return fail(h, CLD_ERR_ARG, "agents_per_scene must be >= 1");
+    if ((int64_t)S * A * N != R) return fail(h, CLD_ERR_ARG, "R=%d != S*A*N = %d*%d*%d", R, S, A, N);
+    return 0;
+  }
+  if (!sc->scene_start || !sc->scene_start_host)
+    return fail(h, CLD_ERR_ARG, "ragged scenes need the offsets twice: scene_start (device) and scene_start_host (host), one is NULL");
+  const int32_t* o = sc->scene_start_host;
+  if (o[0] != 0) return fail(h, CLD_ERR_ARG, "scene_start[0]=%d, must be 0", o[0]);
+  for (int s = 0; s < S; ++s)
+    if (o[s + 1] <= o[s])
+      return fail(h, CLD_ERR_ARG, "scene_start must ascend: scene %d holds %d agents (scene_start[%d]=%d, [%d]=%d), every scene needs >= 1",
+                  s, o[s + 1] - o[s], s, o[s], s + 1, o[s + 1]);
+  if ((int64_t)o[S] * N != R) return fail(h, CLD_ERR_ARG, "scene_start[S]*N = %d*%d != R=%d", o[S], N, R);
+  return 0;
+}
+
 }  // namespace cld
 
 using namespace cld;
@@ -530,6 +551,8 @@ int cld_unicycle(CldHandle* h, const float* curr, const float* u, float* state_o
 int cld_indicators(CldHandle* h, const float* traj, const CldScene* scene, uint8_t* offroad_out, float* coll_out,
                    float* reward_out, int R, void* stream) {
   if (!h || !traj || R < 1) return fail(h, CLD_ERR_ARG, "bad argument");
+  int rc;
+  if (scene && (rc = check_scene(h, scene, R))) return rc;
   return indicators(h, traj, scene, offroad_out, coll_out, reward_out, R, (cudaStream_t)stream);
 }
 
@@ -585,6 +608,7 @@ int cld_guidance_step(CldHandle* h, const float* z_mean, const float* cond, cons
   int rc = check_rows(h, R);
   if (rc) return rc;
   if (!z_mean || !cond || !curr || !scene || !g || !z_out) return fail(h, CLD_ERR_ARG, "null argument");
+  if ((rc = check_scene(h, scene, R))) return rc;
   if ((rc = guidance_prepare_steps(h, g))) return rc;
   if (g->w_map_collision != 0.f && (rc = guidance_prepare_maps(h, scene, (cudaStream_t)stream))) return rc;
   return guidance_step_impl(h, z_mean, cond, nullptr, curr, scene, g, z_out, grad_out, loss_out, R, (cudaStream_t)stream);
@@ -602,6 +626,7 @@ int cld_sample(CldHandle* h, const float* x_init, const float* noises, uint64_t 
   if ((offroad_out || coll_out || g) && !scene) return fail(h, CLD_ERR_ARG, "scene tensors required");
   if (!h->sched.loaded) return fail(h, CLD_ERR_STATE, "schedule not set");
   int rc;
+  if (scene && (rc = check_scene(h, scene, R))) return rc;
   if (g && (rc = guidance_prepare_steps(h, g))) return rc;
   cudaStream_t s = (cudaStream_t)stream;
   const CldConfig& c = h->cfg;
@@ -611,23 +636,34 @@ int cld_sample(CldHandle* h, const float* x_init, const float* noises, uint64_t 
   for (int i = 0; i < n_t; i += stride) steps.push_back(i);
   const int K = (int)steps.size();
   if (x1_valid) *x1_valid = 0;
-  // chunk rows so that whole scenes stay together and the workspace suffices
-  int unit = 1;
+  // chunks of whole scenes, packed greedily in batch order up to max_rows rows: {first scene, first row} of every chunk, then the end
+  std::vector<int> chunk_scene, chunk_row;
   if (scene) {
-    unit = scene->agents_per_scene * scene->num_samp;
-    if (unit < 1 || R % unit) return fail(h, CLD_ERR_ARG, "R=%d is not a multiple of A*N=%d", R, unit);
-    if (R != scene->num_scenes * unit) return fail(h, CLD_ERR_ARG, "R=%d != S*A*N", R);
+    const int S = scene->num_scenes, N = scene->num_samp;
+    auto first_agent = [&](int sidx) { return scene->scene_start ? scene->scene_start_host[sidx] : sidx * scene->agents_per_scene; };
+    for (int sidx = 0; sidx < S; ++sidx) {
+      const int rows = (first_agent(sidx + 1) - first_agent(sidx)) * N;
+      if (rows > c.max_rows) return fail(h, CLD_ERR_ARG, "max_rows=%d is smaller than one scene (scene %d: A*N=%d)", c.max_rows, sidx, rows);
+      if (chunk_scene.empty() || (first_agent(sidx + 1) - first_agent(chunk_scene.back())) * N > c.max_rows) {
+        chunk_scene.push_back(sidx);
+        chunk_row.push_back(first_agent(sidx) * N);
+      }
+    }
+    chunk_scene.push_back(S);
+  } else {
+    for (int r0 = 0; r0 < R; r0 += c.max_rows) chunk_row.push_back(r0);
   }
-  int chunk = (c.max_rows / unit) * unit;
-  if (chunk < unit) return fail(h, CLD_ERR_ARG, "max_rows=%d is smaller than one scene (A*N=%d)", c.max_rows, unit);
-  for (int r0 = 0; r0 < R; r0 += chunk) {
-    const int Rc = (R - r0 < chunk) ? (R - r0) : chunk;
+  chunk_row.push_back(R);
+  for (size_t ci = 0; ci + 1 < chunk_row.size(); ++ci) {
+    const int r0 = chunk_row[ci], Rc = chunk_row[ci + 1] - r0;
     CldScene sub;
     const CldScene* sc = nullptr;
     if (scene) {
       sub = *scene;
       const size_t a0 = (size_t)r0 / scene->num_samp;
-      sub.num_scenes = Rc / unit;
+      sub.num_scenes = chunk_scene[ci + 1] - chunk_scene[ci];
+      // a chunk's offsets keep their values: the kernels subtract scene_start_host[0], its first agent
+      if (sub.scene_start) { sub.scene_start += chunk_scene[ci]; sub.scene_start_host += chunk_scene[ci]; }
       if (sub.extent) sub.extent += a0 * 3;
       if (sub.world_from_agent) sub.world_from_agent += a0 * 9;
       if (sub.raster_from_agent) sub.raster_from_agent += a0 * 9;

@@ -135,6 +135,9 @@ struct CldHandle {
   const void* screen_src = nullptr;        // the drivable_map pointer the screen data belongs to (nullptr: none)
   const uint8_t* screen_pk = nullptr;      // where the screen reads: map_bits or the scene's own packed maps
   int screen_agents = 0, screen_h = 0, screen_w = 0, screen_packed = 0, screen_pitch = 0;
+  // agents of the scene of every agent of the current call (the map-collision term's normalisation), built with the screen data
+  int* scene_size = nullptr;
+  int scene_size_cap = 0, scene_size_agents = 0;
   cudaStream_t aux_stream = nullptr;   // forked from / joined to the caller's stream with the two events below
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   float* ws_loss = nullptr;        // [3, max_rows]
@@ -182,6 +185,12 @@ __host__ __device__ inline size_t stash_index(int layer, int t, int T, int R, in
 }
 constexpr int STASH_V_STRIDE = 64 * 8;   // floats between consecutive values v for the same (row block, unit)
 int fail(CldHandle* h, int code, const char* fmt, ...);
+// agent rows B of a scene; ragged offsets may start above 0 (the scenes of one cld_sample chunk)
+inline int scene_agents(const CldScene* sc) {
+  return sc->scene_start ? sc->scene_start_host[sc->num_scenes] - sc->scene_start_host[0] : sc->num_scenes * sc->agents_per_scene;
+}
+// checks the scene layout a caller passed (num_samp, agents_per_scene or the ragged offsets) against R rows
+int check_scene(CldHandle* h, const CldScene* sc, int R);
 #define CLD_CUDA_OK(h, expr)                                                                   \
   do {                                                                                         \
     cudaError_t _e = (expr);                                                                   \
@@ -281,7 +290,8 @@ int indicators(CldHandle* h, const float* traj, const CldScene* sc, uint8_t* off
 int guidance_loss_grad(CldHandle* h, const float* traj, const CldScene* sc, const CldGuidanceConfig* g,
                        float* dtraj, float* dtraj_map, float* dacc, float* loss, int R, cudaStream_t s);
 // the screen of the map-collision term reads the drivable maps with one bit per pixel: byte-per-pixel maps are packed here, once per
-// cld_sample chunk / cld_guidance_step call (the maps of a call do not change between denoising steps)
+// cld_sample chunk / cld_guidance_step call (the maps of a call do not change between denoising steps); so is the per-agent table of
+// scene sizes the map-collision term normalises by
 int guidance_prepare_maps(CldHandle* h, const CldScene* sc, cudaStream_t s);
 int decode_backward_update(CldHandle* h, const float* z_mean, const float* act, const float* curr,
                            const float* dtraj, const CldGuidanceConfig* g, float* z_out, float* grad_out,

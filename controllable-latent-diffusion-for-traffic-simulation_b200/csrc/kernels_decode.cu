@@ -331,9 +331,8 @@ __global__ void __launch_bounds__(256) indicators_kernel(IndArgs a) {
 int indicators(CldHandle* h, const float* traj, const CldScene* sc, uint8_t* offroad, float* coll, float* reward,
                int R, cudaStream_t s) {
   if (!sc || !sc->raster_from_agent || !sc->drivable_map) return fail(h, CLD_ERR_ARG, "scene tensors missing");
-  if (sc->num_samp < 1 || R != sc->num_scenes * sc->agents_per_scene * sc->num_samp)
-    return fail(h, CLD_ERR_ARG, "R=%d does not match S*A*N=%d*%d*%d", R, sc->num_scenes, sc->agents_per_scene,
-                sc->num_samp);
+  if (sc->num_samp < 1 || R != scene_agents(sc) * sc->num_samp)
+    return fail(h, CLD_ERR_ARG, "R=%d does not match %d agents x N=%d", R, scene_agents(sc), sc->num_samp);
   IndArgs a;
   a.traj = traj; a.rfa = sc->raster_from_agent; a.dmap = sc->drivable_map; a.H = sc->map_h; a.W = sc->map_w; a.packed = sc->map_packed;
   a.others = sc->others_pos; a.avail = sc->others_avail; a.So = sc->num_others;

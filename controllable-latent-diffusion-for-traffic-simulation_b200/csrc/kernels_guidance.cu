@@ -28,7 +28,10 @@ struct LossArgs {
   // time step [B], goal distance [B], per-agent multiplier [B] (A / number of guided agents of the scene: the reference averages over them)
   const float *wp_target, *wp_dist, *wp_w; const int *wp_mode, *wp_time; float w_wp;
   const uint8_t* dmap; int H, W, packed;   // packed: rows of (W + 7) / 8 bytes, pixel x = bit (x & 7) of byte x >> 3
-  int S, A, N, T, R;
+  int S, A, N, T, R;                        // A: agents of every scene, or of the largest one when the scenes are ragged
+  // ragged scenes: scene s holds agents [sstart[s] - sbase, sstart[s + 1] - sbase) of this call (nullptr: s * A ..)
+  const int* sstart; int sbase;
+  const int* scene_size;                    // [B] agents of the scene of every agent (map-collision normalisation)
   float w_ac, w_mc, w_tp;
   int D; float buffer, decay, speed_th, min_target_time;
   int nl, nw;
@@ -127,7 +130,17 @@ constexpr int SCENE_TILE = 64, PARTNER_TILE = 128;
 
 __global__ void __launch_bounds__(512) guidance_loss_grad_kernel(LossArgs a) {
   extern __shared__ __align__(16) float sm[];
-  const int A = a.A, T = a.T, N = a.N;
+  const int T = a.T, N = a.N;
+  const int s = blockIdx.x / N, n = blockIdx.x % N;
+  // agents of this CTA's scene: [ag0, ag0 + A) of the call
+  const int A = a.sstart ? a.sstart[s + 1] - a.sstart[s] : a.A;
+  const size_t ag0 = a.sstart ? (size_t)(a.sstart[s] - a.sbase) : (size_t)s * A;
+  // the agents of a scene are dealt to gridDim.y CTAs (large scenes: 64 agents x 104 steps x 63 partners would otherwise sit on
+  // S * N CTAs); every CTA visits the poses of ALL agents (the partners) and evaluates the terms of agents [i_lo, i_hi).  The
+  // split is laid out for a.A agents, the largest scene: a CTA past the end of a smaller scene has nothing to do.
+  const int per_cta = (a.A + (int)gridDim.y - 1) / (int)gridDim.y;
+  const int i_lo = (int)blockIdx.y * per_cta, i_hi = min(A, i_lo + per_cta);
+  if (i_lo >= A) return;
   // The partners j of the agent-collision term pass through shared memory in tiles.  A scene of at most SCENE_TILE agents is
   // one tile holding all its steps, staged once.  A larger scene is streamed as tiles of PARTNER_TILE partners x the 32 steps
   // of one lane slot, so shared memory does not depend on A.  Tiles go in ascending j: every sum over partners is added in the
@@ -137,14 +150,8 @@ __global__ void __launch_bounds__(512) guidance_loss_grad_kernel(LossArgs a) {
   float* pose = sm;                         // [P][TS][4] world Px, Py, cos(Psi), sin(Psi) of the tile's partners
   float* agt = pose + (size_t)P * TS * 4;   // [P][8]: rad, cmin, cmax, moving, R00, R01, R10, R11
   float* wts = agt + P * 8;                 // [T] decay weights
-  const int s = blockIdx.x / N, n = blockIdx.x % N;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int nthr = blockDim.x, nwarps = nthr >> 5;       // 16 warps: one agent per warp at 16 agents per scene (latency-bound loops: more warps per SM)
-  // the agents of a scene are dealt to gridDim.y CTAs (large scenes: 64 agents x 104 steps x 63 partners would otherwise sit on
-  // S * N CTAs); every CTA visits the poses of ALL agents (the partners) and evaluates the terms of agents [i_lo, i_hi)
-  const int per_cta = (A + (int)gridDim.y - 1) / (int)gridDim.y;
-  const int i_lo = (int)blockIdx.y * per_cta, i_hi = min(A, i_lo + per_cta);
-  const size_t ag0 = (size_t)s * A;
   const float inv_AN = 1.0f / (float)(A * N);
 
   for (int t = tid; t < T; t += nthr) wts[t] = a.wts[t];
@@ -592,7 +599,7 @@ __global__ void __launch_bounds__(256) guidance_map_list_kernel(LossArgs a) {
     }
     if (lane == 0) {
       const float wt = a.wts[t];
-      float kk = a.w_mc * (1.0f / (float)(a.A * N)) * wt;
+      float kk = a.w_mc * (1.0f / (float)(__ldg(a.scene_size + g) * N)) * wt;
       float4* o = reinterpret_cast<float4*>(a.dtraj) + item;
       if (a.assign) {
         *o = make_float4(kk * gx, kk * gy, 0.f, kk * gpsi);
@@ -618,10 +625,37 @@ static float host_linspace(float lo, float hi, int n, int i) {
   return (i < n / 2) ? lo + step * (float)i : hi - step * (float)(n - 1 - i);
 }
 
+// agents of the scene of every agent g < B of a call: the last scene whose first agent is <= g (ragged), or A
+__global__ void __launch_bounds__(256) guidance_scene_size_kernel(const int* __restrict__ sstart, int sbase, int S, int A, int B,
+                                                                  int* __restrict__ out) {
+  const int g = blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= B) return;
+  if (!sstart) { out[g] = A; return; }
+  int lo = 0, hi = S - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (sstart[mid] - sbase <= g) lo = mid; else hi = mid - 1;
+  }
+  out[g] = sstart[lo + 1] - sstart[lo];
+}
+
 int guidance_prepare_maps(CldHandle* h, const CldScene* sc, cudaStream_t s) {
   h->screen_src = nullptr;
-  if (!sc || !sc->drivable_map || sc->map_w < 1 || sc->map_h < 1) return 0;     // no screen: every moving item takes the full path
-  const int n_maps = sc->num_scenes * sc->agents_per_scene;
+  h->scene_size_agents = 0;
+  if (!sc) return 0;
+  const int n_maps = scene_agents(sc);
+  if (n_maps > h->scene_size_cap) {
+    // grows like map_bits: only when a call with more agents arrives
+    int* p = nullptr;
+    CLD_CUDA_OK(h, cudaMalloc((void**)&p, (size_t)n_maps * sizeof(int)));
+    h->allocs.push_back(p);
+    h->scene_size = p; h->scene_size_cap = n_maps;
+  }
+  guidance_scene_size_kernel<<<(n_maps + 255) / 256, 256, 0, s>>>(sc->scene_start, sc->scene_start ? sc->scene_start_host[0] : 0,
+                                                                 sc->num_scenes, sc->agents_per_scene, n_maps, h->scene_size);
+  CLD_LAUNCH_OK(h, "guidance_scene_size_kernel");
+  h->scene_size_agents = n_maps;
+  if (!sc->drivable_map || sc->map_w < 1 || sc->map_h < 1) return 0;     // no screen: every moving item takes the full path
   if (sc->map_packed) {
     h->screen_pk = sc->drivable_map; h->screen_pitch = (sc->map_w + 7) / 8;
   } else {
@@ -664,9 +698,21 @@ int guidance_loss_grad(CldHandle* h, const float* traj, const CldScene* sc, cons
                        float* dtraj_map, float* dacc, float* loss, int R, cudaStream_t s) {
   if (!sc || !g) return fail(h, CLD_ERR_ARG, "scene / guidance config missing");
   int rc;
-  const int S = sc->num_scenes, A = sc->agents_per_scene, N = sc->num_samp, T = h->cfg.horizon;
-  if (R != S * A * N) return fail(h, CLD_ERR_ARG, "R=%d does not match S*A*N=%d*%d*%d", R, S, A, N);
-  if (A < 1) return fail(h, CLD_ERR_UNSUPPORTED, "agents_per_scene must be >= 1");
+  const int S = sc->num_scenes, N = sc->num_samp, T = h->cfg.horizon;
+  if (!sc->scene_start && sc->agents_per_scene < 1) return fail(h, CLD_ERR_UNSUPPORTED, "agents_per_scene must be >= 1");
+  if (S < 1 || N < 1 || R != scene_agents(sc) * N) return fail(h, CLD_ERR_ARG, "R=%d does not match %d agents x N=%d", R, scene_agents(sc), N);
+  // launch geometry: the largest scene (A), the largest one that is staged as one tile, and whether any is streamed in tiles
+  int A = sc->agents_per_scene, A_tile = A <= SCENE_TILE ? A : 0;
+  bool any_streamed = A > SCENE_TILE;
+  if (sc->scene_start) {
+    A = A_tile = 0;
+    any_streamed = false;
+    for (int i = 0; i < S; ++i) {
+      const int n = sc->scene_start_host[i + 1] - sc->scene_start_host[i];
+      A = n > A ? n : A;
+      if (n <= SCENE_TILE) A_tile = n > A_tile ? n : A_tile; else any_streamed = true;
+    }
+  }
   if (g->num_disks < 1 || g->num_disks > 5) return fail(h, CLD_ERR_UNSUPPORTED, "num_disks must be in [1,5]");
   if (g->num_points_l < 1 || g->num_points_l > 16 || g->num_points_w < 1 || g->num_points_w > 16 ||
       g->num_points_l * g->num_points_w > 128)
@@ -679,6 +725,10 @@ int guidance_loss_grad(CldHandle* h, const float* traj, const CldScene* sc, cons
   a.extent = sc->extent; a.wfa = sc->world_from_agent; a.rfa = sc->raster_from_agent; a.speed = sc->curr_speed;
   a.target = sc->target_pos; a.dmap = sc->drivable_map; a.H = sc->map_h; a.W = sc->map_w; a.packed = sc->map_packed;
   a.S = S; a.A = A; a.N = N; a.T = T; a.R = R;
+  a.sstart = sc->scene_start; a.sbase = sc->scene_start ? sc->scene_start_host[0] : 0;
+  a.scene_size = h->scene_size;
+  if (g->w_map_collision != 0.f && h->scene_size_agents != R / N)
+    return fail(h, CLD_ERR_STATE, "internal: the per-agent scene sizes of the map-collision term were not prepared for this call");
   a.w_ac = g->w_agent_collision; a.w_mc = g->w_map_collision; a.w_tp = g->w_target_pos;
   a.tspeed = sc->target_speed; a.w_ts = g->w_target_speed; a.w_al = g->w_acc_limit; a.acc_limit = g->acc_limit;
   a.w_sl = g->w_speed_limit; a.speed_limit = g->speed_limit; a.dacc = a.w_al != 0.f ? dacc : nullptr;
@@ -689,7 +739,7 @@ int guidance_loss_grad(CldHandle* h, const float* traj, const CldScene* sc, cons
   if (a.w_al != 0.f && !dacc) return fail(h, CLD_ERR_STATE, "internal: acc-limit guidance without a d(acc) buffer");
   a.work = h->map_work; a.assign = 0; a.exhaustive = h->env_map_exhaustive ? 1 : 0;
   // the screen data belongs to the maps guidance_prepare_maps last saw
-  const bool screen_ok = h->screen_src == (const void*)sc->drivable_map && h->screen_agents >= S * A && h->screen_h == sc->map_h &&
+  const bool screen_ok = h->screen_src == (const void*)sc->drivable_map && h->screen_agents >= R / N && h->screen_h == sc->map_h &&
                          h->screen_w == sc->map_w && h->screen_packed == sc->map_packed;
   a.pk = screen_ok ? h->screen_pk : nullptr; a.pk_pitch = h->screen_pitch;
   a.D = g->num_disks; a.buffer = g->buffer_dist; a.decay = g->decay_rate; a.speed_th = g->speed_th;
@@ -705,9 +755,11 @@ int guidance_loss_grad(CldHandle* h, const float* traj, const CldScene* sc, cons
     for (int t = 0; t < T; ++t) a.wts[t] /= sum;
     for (int t = T; t < CLD_MAX_T; ++t) a.wts[t] = 0.f;
   }
-  // the whole scene (at most 133 KB: A = 64, T = 128), or one tile of partners (65 KB and the decay weights)
+  // the whole scene (at most 133 KB: A = 64, T = 128), or one tile of partners (65 KB and the decay weights), whichever of the
+  // two the scenes of the call need more of
   const bool one_tile = A <= SCENE_TILE;
-  const size_t smem = ((size_t)(one_tile ? A : PARTNER_TILE) * ((one_tile ? T : 32) * 4 + 8) + T) * sizeof(float);
+  const size_t tile_floats = (size_t)A_tile * (T * 4 + 8), stream_floats = any_streamed ? (size_t)PARTNER_TILE * (32 * 4 + 8) : 0;
+  const size_t smem = ((tile_floats > stream_floats ? tile_floats : stream_floats) + T) * sizeof(float);
   CLD_CUDA_OK(h, cudaFuncSetAttribute(guidance_loss_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const bool fork = dtraj_map != nullptr && loss == nullptr && a.w_mc != 0.f;
   if (fork) {
@@ -725,7 +777,8 @@ int guidance_loss_grad(CldHandle* h, const float* traj, const CldScene* sc, cons
     if ((rc = launch_map(h, am, h->aux_stream))) return rc;
     CLD_CUDA_OK(h, cudaEventRecord(h->ev_join, h->aux_stream));
   }
-  // enough CTAs for ~2 per SM: the agents of a scene are split over gridDim.y CTAs when there are few (scene, sample) pairs
+  // enough CTAs for ~2 per SM: the agents of a scene are split over gridDim.y CTAs when there are few (scene, sample) pairs.  The
+  // split and the warps per CTA are chosen for the largest scene; with several tiles a CTA still holds at most one agent per warp.
   int split = 1;
   if (one_tile) {
     while (S * N * split < 2 * h->num_sms && split * 2 <= (A + 3) / 4) split *= 2;

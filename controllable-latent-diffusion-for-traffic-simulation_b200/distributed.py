@@ -11,6 +11,8 @@ B200 box, gloo in the CPU tests).  Nothing here computes: it slices, packs and g
 import torch
 import torch.distributed as dist
 
+from .keys import scene_size_list, scene_sizes
+
 # data_batch / aux_info entries indexed by agent row (B = S*A, scene-major)
 PER_AGENT_KEYS = (
     "extent", "world_from_agent", "raster_from_agent", "curr_speed", "drivable_map", "drivable_map_bits", "scene_index", "target_pos", "target_speed",
@@ -30,13 +32,14 @@ def shard_scenes(num_scenes, world_size, rank):
 
 
 def shard_batch(batch, agents_per_scene, world_size, rank):
-    """Slice every per-agent tensor of a data_batch / aux_info dict to this rank's scenes."""
+    """Slice every per-agent tensor of a data_batch / aux_info dict to this rank's scenes (whole scenes, `shard_scenes`).
+    agents_per_scene: an int, the list of scene sizes of a ragged batch, or None to read the sizes from batch["scene_index"]."""
     some = next(v for k, v in batch.items() if k in PER_AGENT_KEYS and torch.is_tensor(v))
     B = some.shape[0]
-    if B % agents_per_scene:
-        raise ValueError("B=%d is not a multiple of agents_per_scene=%d" % (B, agents_per_scene))
-    s0, s1 = shard_scenes(B // agents_per_scene, world_size, rank)
-    a0, a1 = s0 * agents_per_scene, s1 * agents_per_scene
+    sizes = scene_sizes(batch.get("scene_index"), B) if agents_per_scene is None else scene_size_list(agents_per_scene, B)
+    s0, s1 = shard_scenes(len(sizes), world_size, rank)
+    a0 = sum(sizes[:s0])
+    a1 = a0 + sum(sizes[s0:s1])
     out = {}
     for k, v in batch.items():
         out[k] = v[a0:a1] if (k in PER_AGENT_KEYS and torch.is_tensor(v) and v.shape[0] == B) else v

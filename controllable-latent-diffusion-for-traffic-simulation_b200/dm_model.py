@@ -12,13 +12,14 @@ Extra keyword arguments of `forward` (all default to the reference behaviour):
   guidance=  dict of guidance weights (engine.default_guidance) + data_batch scene tensors
   seed=      Philox seed for in-kernel noise when `noise` is None and use_device_rng=True
 """
+import bisect
 import math
 
 import numpy as np
 import torch
 import torch.nn as nn
 
-from .keys import agents_per_scene as _agents_per_scene, scene_buckets as _scene_buckets, scene_sizes as _scene_sizes
+from .keys import scene_size_list as _scene_size_list, scene_sizes as _scene_sizes
 
 
 class _Slot(nn.Module):
@@ -294,23 +295,15 @@ class DmModel(nn.Module):
         rep = (lambda v: v.repeat_interleave(N, dim=0)) if N > 1 else (lambda v: v)
         cond_rows = rep(cond)
         curr_rows = rep(aux_info['curr_states']) if 'curr_states' in aux_info else None
-        A, buckets = agents_per_scene, None
-        if guidance is not None or want_indicators:
-            if A is None:
-                sizes = _scene_sizes(data_batch.get('scene_index'), B)
-                if len(set(sizes)) > 1:
-                    buckets = _scene_buckets(sizes)
-                else:
-                    A = sizes[0]
-            elif B % A:
-                raise ValueError("B=%d agents is not a multiple of agents_per_scene=%d" % (B, A))
+        # agents of every scene, in batch order (None: the scene structure does not matter to an unguided call)
+        sizes = None
+        if agents_per_scene is not None:
+            sizes = _scene_size_list(agents_per_scene, B)
+        elif guidance is not None or want_indicators:
+            sizes = _scene_sizes(data_batch.get('scene_index'), B)
         dev_seed = (seed or 0) if use_device_rng else 0
-        if buckets is not None:
-            out = self._sample_ragged(buckets, data_batch, B, N, x_init, cond_rows, curr_rows, noise, dev_seed, guidance, sampler,
-                                      want_traj, want_indicators, row_offset)
-        else:
-            out = self._sample_uniform(eng, data_batch, B, A, N, x_init, cond_rows, curr_rows, noise, dev_seed, guidance, sampler,
-                                       want_traj, want_indicators, row_offset)
+        out = self._sample_scenes(eng, data_batch, B, sizes, N, x_init, cond_rows, curr_rows, noise, dev_seed, guidance, sampler,
+                                  want_traj, want_indicators, row_offset)
         log_prob_final = None
         if 0 in steps and sampler == "ddpm":
             # x0 == mean at t == 0, so Normal(mean, sigma).log_prob(x0) is constant (dm_model.py:128-132)
@@ -330,65 +323,43 @@ class DmModel(nn.Module):
             res['coll'] = out['coll']
         return res
 
-    def _sample_uniform(self, eng, data_batch, B, A, N, x_init, cond_rows, curr_rows, noise, dev_seed, guidance, sampler, want_traj,
-                        want_indicators, row_offset):
-        """One call of the sampler for a batch whose scenes all hold A agents (or whose scene structure does not matter)."""
-        n_lanes = min(self._lanes, B // A) if (A and self._lanes > 1) else 1
+    def _sample_scenes(self, eng, data_batch, B, sizes, N, x_init, cond_rows, curr_rows, noise, dev_seed, guidance, sampler, want_traj,
+                       want_indicators, row_offset):
+        """One call of the sampler (one per lane) for a batch of scenes of `sizes` agents, uniform or ragged."""
+        n_lanes = min(self._lanes, len(sizes)) if (sizes and self._lanes > 1) else 1
         if n_lanes > 1:
-            return self._sample_lanes(n_lanes, data_batch, B, A, N, x_init, cond_rows, curr_rows, noise, dev_seed, guidance,
+            return self._sample_lanes(n_lanes, data_batch, B, sizes, N, x_init, cond_rows, curr_rows, noise, dev_seed, guidance,
                                       sampler, want_traj, want_indicators, row_offset)
-        scene = eng.make_scene(data_batch, B // A, A, N) if (guidance is not None or want_indicators) else None
+        scene = (eng.make_scene(data_batch, len(sizes), sizes[0], N, scene_sizes=sizes)
+                 if (guidance is not None or want_indicators) else None)
         return eng.sample(x_init, cond_rows, noises=noise, seed=dev_seed, row_offset=row_offset, curr_rows=curr_rows, scene=scene,
                           guidance=guidance, stride=self.stride, sampler=sampler, want_traj=want_traj, want_indicators=want_indicators)
 
-    def _sample_ragged(self, buckets, data_batch, B, N, x_init, cond_rows, curr_rows, noise, dev_seed, guidance, sampler, want_traj,
-                       want_indicators, row_offset):
-        """Scenes of different sizes: one uniform sub-batch per distinct scene size (`keys.scene_buckets`), results scattered back
-        into batch order.  Scenes never interact, so this equals sampling every scene on its own.  With pre-drawn `x_init` / `noise`
-        every row gets its own draw whatever the bucketing; the in-kernel Philox generator is keyed by the row's position in the
-        bucketed order (deterministic for a given batch composition, but not the id the row has in `data_batch`)."""
-        device = self.betas.device
-        out, pos = None, 0
-        for A, idx in buckets:
-            idx = idx.to(device)
-            rows = (idx[:, None] * N + torch.arange(N, device=device)[None, :]).reshape(-1)
-            nb = idx.numel()
-            sub = {k: (v.index_select(0, idx.to(v.device)) if (torch.is_tensor(v) and v.dim() > 0 and v.shape[0] == B) else v)
-                   for k, v in data_batch.items()}
-            sub['scene_index'] = torch.arange(nb // A, device=device).repeat_interleave(A)
-            sel = lambda v: None if v is None else v.index_select(0, rows.to(v.device))                  # noqa: E731
-            o = self._sample_uniform(self.engine(nb * N), sub, nb, A, N, sel(x_init), sel(cond_rows), sel(curr_rows),
-                                     None if noise is None else noise.index_select(1, rows.to(noise.device)), dev_seed, guidance,
-                                     sampler, want_traj, want_indicators, row_offset + pos)
-            pos += nb * N
-            if out is None:
-                out = {k: (None if v is None else v.new_empty((B * N,) + tuple(v.shape[1:]))) for k, v in o.items()}
-            for k, v in o.items():
-                if v is None:
-                    out[k] = None
-                elif out[k] is not None:
-                    out[k].index_copy_(0, rows.to(v.device), v)
-        return out
-
-    def _sample_lanes(self, n_lanes, data_batch, B, A, N, x_init, cond_rows, curr_rows, noise, dev_seed, guidance, sampler,
+    def _sample_lanes(self, n_lanes, data_batch, B, sizes, N, x_init, cond_rows, curr_rows, noise, dev_seed, guidance, sampler,
                       want_traj, want_indicators, row_offset=0):
-        """Scenes split into `n_lanes` contiguous whole-scene sub-batches, each sampled by its own engine on its own stream
-        (scenes never interact and in-kernel Philox noise is indexed by the global row id, so the result equals the
+        """Scenes split into `n_lanes` contiguous groups of whole scenes, balanced by rows, each sampled by its own engine on its
+        own stream (scenes never interact and in-kernel Philox noise is indexed by the global row id, so the result equals the
         single-lane one bit for bit)."""
         device = self.betas.device
-        S = B // A
+        cum = [0]
+        for c in sizes:
+            cum.append(cum[-1] + c)
+        # lane li ends after the last scene that ends at or before li / n_lanes of the agents
+        scaled = [c * n_lanes for c in cum]
+        cut = [bisect.bisect_right(scaled, B * li) - 1 for li in range(n_lanes + 1)]
         cur = torch.cuda.current_stream(device)
         parts = []
         for li in range(n_lanes):
-            s0, s1 = S * li // n_lanes, S * (li + 1) // n_lanes
+            s0, s1 = cut[li], cut[li + 1]
             if s1 == s0:
                 continue
-            b0, b1, r0, r1 = s0 * A, s1 * A, s0 * A * N, s1 * A * N
+            b0, b1, r0, r1 = cum[s0], cum[s1], cum[s0] * N, cum[s1] * N
             eng, st = self._lane_engine(li, r1 - r0)
             st.wait_stream(cur)
             with torch.cuda.stream(st):
                 sub = {k: (v[b0:b1] if (torch.is_tensor(v) and v.dim() > 0 and v.shape[0] == B) else v) for k, v in data_batch.items()}
-                scene = eng.make_scene(sub, s1 - s0, A, N) if (guidance is not None or want_indicators) else None
+                scene = (eng.make_scene(sub, s1 - s0, sizes[s0], N, scene_sizes=sizes[s0:s1])
+                         if (guidance is not None or want_indicators) else None)
                 o = eng.sample(None if x_init is None else x_init[r0:r1], cond_rows[r0:r1], noises=None if noise is None else noise[:, r0:r1],
                                seed=dev_seed, row_offset=row_offset + r0, curr_rows=None if curr_rows is None else curr_rows[r0:r1],
                                scene=scene, guidance=guidance, stride=self.stride, sampler=sampler, want_traj=want_traj,

@@ -149,9 +149,12 @@ class Engine:
 
     # ------------------------------------------------------------------ scene / guidance structs
     @_on_device
-    def make_scene(self, batch, num_scenes, agents_per_scene, num_samp):
+    def make_scene(self, batch, num_scenes, agents_per_scene, num_samp, scene_sizes=None):
         """batch: the reference's data_batch dict (extent, world_from_agent, raster_from_agent, curr_speed,
-        drivable_map, [target_pos], [all_other_agents_future_positions/_availability])."""
+        drivable_map, [target_pos], [all_other_agents_future_positions/_availability]).
+        scene_sizes: agents of every scene (`keys.scene_sizes`), in batch order; agents_per_scene is then ignored.  Scenes of
+        different sizes are passed as offsets (CldScene.scene_start), equal sizes as agents_per_scene.  None: every scene holds
+        agents_per_scene agents."""
         d = self.device
         # the drivable map may arrive bit-packed ("drivable_map_bits" [B,H,W/8] uint8, synthetic.pack_drivable_map): 1/8 of the bytes
         bits = batch.get("drivable_map_bits")
@@ -184,6 +187,16 @@ class Engine:
             raise ValueError("target_speed must be [B, T=%d]" % self.T)
         if keep["others"] is not None and keep["others"].shape[2] != self.T:
             raise ValueError("all_other_agents_future_positions must cover the horizon T=%d" % self.T)
+        sizes = None if scene_sizes is None else [int(c) for c in scene_sizes]
+        if sizes is not None and len(sizes) != int(num_scenes):
+            raise ValueError("%d scene sizes for num_scenes=%d" % (len(sizes), num_scenes))
+        if sizes is not None and len(set(sizes)) == 1:
+            sc.agents_per_scene = sizes[0]
+        elif sizes is not None:
+            # the library takes the offsets twice: on the device for the kernels, on the host for checks and chunking
+            host = torch.tensor([0] + sizes, dtype=torch.int32).cumsum(0, dtype=torch.int32).contiguous()
+            keep["scene_start_host"], keep["scene_start"] = host, host.to(d)
+            sc.scene_start, sc.scene_start_host = _ptr(keep["scene_start"]), _ptr(host)
         sc._keep = keep
         return sc
 

@@ -40,11 +40,26 @@ def scene_sizes(scene_index, B):
     return [int(c) for c in counts.tolist()]
 
 
+def scene_size_list(agents_per_scene, B):
+    """Agents of every scene of B agent rows: `agents_per_scene` is an int (uniform scenes, B must be a multiple) or a list of
+    scene sizes in batch order (ragged scenes, summing to B)."""
+    import numbers
+    if isinstance(agents_per_scene, numbers.Integral):
+        A = int(agents_per_scene)
+        if A < 1 or B % A:
+            raise ValueError("B=%d agents is not a multiple of agents_per_scene=%d" % (B, A))
+        return [A] * (B // A)
+    sizes = [int(c) for c in agents_per_scene]
+    if not sizes or min(sizes) < 1 or sum(sizes) != B:
+        raise ValueError("scene sizes must be >= 1 and sum to B=%d (got %d scenes, %d agents)" % (B, len(sizes), sum(sizes)))
+    return sizes
+
+
 def scene_buckets(sizes):
-    """Ragged batches (the reference builds a block-diagonal scene mask from `scene_index`, guidance_loss.py:493-503, and accepts
-    scenes of different sizes): the kernels index rows as (scene * A + agent) * N + sample with ONE A per call, so a ragged batch is
-    sampled as one uniform sub-batch per distinct scene size.  Returns [(A, agent_index LongTensor)], sizes ascending; the agent
-    indices of a bucket are scene-major in batch order."""
+    """Groups the scenes of a ragged batch (the reference builds a block-diagonal scene mask from `scene_index`,
+    guidance_loss.py:493-503, and accepts scenes of different sizes) by size: one uniform sub-batch per distinct scene size.
+    Returns [(A, agent_index LongTensor)], sizes ascending; the agent indices of a bucket are scene-major in batch order.  (The
+    sampler takes a ragged batch in one call; this grouping is what a caller of a uniform-only interface would do.)"""
     import torch
     starts, pos = [], 0
     for c in sizes:
@@ -58,7 +73,7 @@ def scene_buckets(sizes):
 
 
 def agents_per_scene(scene_index, B):
-    """Number of agents A of every scene of a UNIFORM batch, checked (ragged batches: `scene_buckets`)."""
+    """Number of agents A of every scene of a UNIFORM batch, checked (ragged batches: `scene_sizes`)."""
     import torch
     if scene_index is None:
         return int(B)

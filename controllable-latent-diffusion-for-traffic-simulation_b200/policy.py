@@ -4,24 +4,39 @@ directly on the sampling path -- `DiffuserTrafficModel.get_action` (src/tbsim/al
 with the smallest (unweighted, summed) guidance loss is chosen -- per SCENE when a scene-level term (agent_collision) is active,
 per agent otherwise -- and stationary agents are zeroed.  The simulator / trajdata environment around it is out of scope.
 """
+import numbers
+
 import torch
 
-from .keys import agents_per_scene as _agents_per_scene, default_guidance
+from .keys import default_guidance, scene_size_list, scene_sizes
 
 SCENE_LEVEL_TERMS = ("agent_collision",)      # + social_group / gpt* in the reference, which are not built
 LOSS_ROWS = ("agent_collision", "map_collision", "target_pos", "target_speed", "acc_limit", "speed_limit", "waypoint")
 
 
 def choose_action_from_guidance(guide_losses, agents_per_scene, scene_level):
-    """guide_losses [B, N, G] (B = S * A agents, N samples, G active terms, NaN = not applicable) -> act_idx [B].
+    """guide_losses [B, N, G] (B agents, N samples, G active terms, NaN = not applicable) -> act_idx [B].  agents_per_scene: an
+    int (B = S * A) or the list of scene sizes of a ragged batch.
     scene_level: argmin over samples of the loss summed over the agents of the scene (guidance_loss.py:50-56), else per agent."""
     B, N, _ = guide_losses.shape
     tot = torch.nansum(guide_losses, dim=-1)                                  # [B, N]
-    if scene_level:
-        S = B // agents_per_scene
-        idx = torch.argmin(tot.reshape(S, agents_per_scene, N).sum(dim=1), dim=1)   # [S]
-        return idx.repeat_interleave(agents_per_scene)
-    return torch.argmin(tot, dim=-1)
+    if not scene_level:
+        return torch.argmin(tot, dim=-1)
+    if not isinstance(agents_per_scene, numbers.Integral):
+        # segment sums: the scenes of one size are summed as one uniform batch, so every scene's sum is the one a call on that
+        # scene alone computes
+        sizes = scene_size_list(agents_per_scene, B)
+        starts = torch.tensor([0] + sizes[:-1]).cumsum(0)
+        idx = torch.empty(B, dtype=torch.long, device=tot.device)
+        for A in sorted(set(sizes)):
+            first = starts[torch.tensor(sizes) == A]
+            rows = (first[:, None] + torch.arange(A)[None, :]).reshape(-1).to(tot.device)
+            pick = torch.argmin(tot.index_select(0, rows).reshape(-1, A, N).sum(dim=1), dim=1)
+            idx[rows] = pick.repeat_interleave(A)
+        return idx
+    S = B // agents_per_scene
+    idx = torch.argmin(tot.reshape(S, agents_per_scene, N).sum(dim=1), dim=1)   # [S]
+    return idx.repeat_interleave(agents_per_scene)
 
 
 class GuidedDiffusionPolicy:
@@ -39,7 +54,9 @@ class GuidedDiffusionPolicy:
         guide_losses {term: [B,N]}})."""
         B = obs_dict["history_positions"].shape[0]
         N = int(num_action_samples)
-        A = _agents_per_scene(obs_dict.get("scene_index"), B)
+        sizes = scene_sizes(obs_dict.get("scene_index"), B)
+        # a uniform batch keeps the integer form (its scene-level choice is one reshape)
+        A = sizes[0] if len(set(sizes)) == 1 else sizes
         if aux_info is None:
             if self.context_encoder is None:
                 raise ValueError("get_action needs aux_info (cond_feat, curr_states) or a context encoder")
@@ -61,7 +78,7 @@ class GuidedDiffusionPolicy:
             g = dict(default_guidance(), **self.guidance)
             g["grad_steps"] = 1
             eng = self.dm.engine(B * N)
-            scene = eng.make_scene(obs_dict, B // A, A, N)
+            scene = eng.make_scene(obs_dict, len(sizes), sizes[0], N, scene_sizes=sizes)
             rep = (lambda v: v.repeat_interleave(N, dim=0)) if N > 1 else (lambda v: v)
             _, _, per = eng.guidance_step(out["pred_traj"], rep(aux_info["cond_feat"]), rep(aux_info["curr_states"]), scene, g)
             active = [k for k in LOSS_ROWS if float(g.get(k, 0.0)) != 0.0]

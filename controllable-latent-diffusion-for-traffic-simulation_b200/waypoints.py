@@ -4,7 +4,7 @@
 The reference's `forward()` is two things: host logic that turns WORLD targets into a per-agent (local target, branch) -- exact vs
 progress, target time passed, `have_reached_mask` -- and one of four per-agent formulas.  The formulas and their analytic gradients are
 in the guidance kernel (`CldScene.wp_*`, `CldGuidanceConfig.w_waypoint`); the classes here reproduce the host logic on device tensors and
-hand the kernel its five per-agent arrays through `scene_entries()`, which is merged into the `data_batch`:
+hand the kernel its five per-agent arrays through `scene_entries()`, which is merged into the `data_batch` (`agents_per_scene`: an int, or the scene sizes of a ragged batch):
 
     term = GlobalTargetPosAtTime(target_pos_world, target_time, urgency, pref_speed, dt=0.1, target_tolerance=2, action_num=5)
     term.update(global_t)                                  # GuidanceLoss.update (guidance_loss.py:196-202)
@@ -14,7 +14,11 @@ hand the kernel its five per-agent arrays through `scene_entries()`, which is me
 `have_reached` is kept per agent across calls like the reference's `have_reached_mask`.  The reference averages a term over the guided
 agents only (`agt_mask`, guidance_loss.py:2159-2172): `wp_weight` = A / (guided agents of the scene) restores that under the kernel's 1 / (A N).
 """
+import numbers
+
 import torch
+
+from .keys import scene_size_list
 
 
 def _tf_points(pts, mat):
@@ -23,9 +27,17 @@ def _tf_points(pts, mat):
 
 
 def _weights(mode, agents_per_scene):
-    act = (mode != 0).float().view(-1, agents_per_scene)
-    k = act.sum(dim=1, keepdim=True).clamp(min=1.0)
-    return (act * (agents_per_scene / k)).reshape(-1)
+    """A / (guided agents of the scene) for the guided agents, 0 for the others; agents_per_scene: an int or the scene sizes of a
+    ragged batch."""
+    if isinstance(agents_per_scene, numbers.Integral):
+        act = (mode != 0).float().view(-1, agents_per_scene)
+        k = act.sum(dim=1, keepdim=True).clamp(min=1.0)
+        return (act * (agents_per_scene / k)).reshape(-1)
+    sizes = torch.tensor(scene_size_list(agents_per_scene, mode.shape[0]), device=mode.device)
+    seg = torch.repeat_interleave(torch.arange(sizes.numel(), device=mode.device), sizes)
+    act = (mode != 0).float()
+    k = torch.zeros(sizes.numel(), device=mode.device).index_add_(0, seg, act).clamp(min=1.0)   # counts: exact in any order
+    return act * (k.reciprocal() * sizes.float())[seg]          # how torch evaluates the int form's `A / k`
 
 
 class TargetPosAtTime:

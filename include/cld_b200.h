@@ -9,7 +9,8 @@
  *
  * Conventions
  *   - plain pointers and sizes only; every data pointer is a DEVICE pointer owned by the caller
- *     (e.g. torch.Tensor.data_ptr()), contiguous, fp32 unless stated;
+ *     (e.g. torch.Tensor.data_ptr()), contiguous, fp32 unless stated -- except the HOST arrays of
+ *     cld_set_schedule and CldScene.scene_start_host;
  *   - `stream` is a cudaStream_t passed as void*; all work is enqueued asynchronously on it, no
  *     implicit synchronisation, no allocation in the step path (CUDA-graph capturable);
  *   - return 0 on success, a negative CldStatus otherwise; cld_last_error() gives the message;
@@ -17,7 +18,8 @@
  *   - there is NO CPU fallback and no other-architecture dispatch: cld_create fails on a device
  *     that is not compute capability 10.x.
  *   - row layout: R = S*A*N rows, row = (scene*A + agent)*N + sample  (the reference's
- *     TensorUtils.join_dimensions of [B,N,...], models/dm/dm_model.py:110).
+ *     TensorUtils.join_dimensions of [B,N,...], models/dm/dm_model.py:110); ragged scenes
+ *     (CldScene.scene_start): R = B*N, row = (scene_start[scene] + agent)*N + sample.
  */
 #ifndef CLD_B200_H_
 #define CLD_B200_H_
@@ -88,10 +90,10 @@ typedef struct {
   int32_t grad_steps;       /* optimizer iterations per guided step (perturb's grad_steps); 0 and 1 both mean one, < 0 is CLD_ERR_ARG */
 } CldGuidanceConfig;
 
-/* Per-agent scene tensors (the reference's data_batch entries), B = S*A agent rows, scene-major. */
+/* Per-agent scene tensors (the reference's data_batch entries), B = S*A agent rows (ragged: scene_start[S]), scene-major. */
 typedef struct {
   int32_t num_scenes;               /* S */
-  int32_t agents_per_scene;         /* A >= 1; any size is guided: one scene's A*N rows must fit CldConfig.max_rows */
+  int32_t agents_per_scene;         /* A >= 1 (ignored with scene_start); any size is guided: one scene's A*N rows must fit CldConfig.max_rows */
   int32_t num_samp;                 /* N */
   const float* extent;              /* [B,3]  data_batch['extent']                               */
   const float* world_from_agent;    /* [B,3,3]                                                   */
@@ -114,6 +116,13 @@ typedef struct {
   const int32_t* wp_time;           /* [B]   or NULL */
   const float* wp_dist;             /* [B]   or NULL */
   const float* wp_weight;           /* [B]   or NULL */
+  /* ragged batches: NULL = every scene holds agents_per_scene agents; otherwise agents_per_scene is ignored and scene s holds agent rows
+   * [scene_start[s], scene_start[s+1]): S+1 ascending int32 offsets, [0] = 0, [S] = B, every scene >= 1 agent.
+   * Given twice: on the DEVICE for the kernels, and on the HOST for validation, chunking and launch geometry (read during the call only).
+   * scene_start_host is the one HOST pointer of this struct, an exception to the device-pointer convention above.
+   * cld_sample, cld_guidance_step and cld_indicators take ragged scenes; each scene is guided as if it were alone in the call. */
+  const int32_t* scene_start;
+  const int32_t* scene_start_host;
 } CldScene;
 
 int cld_version(void);
